@@ -1,9 +1,17 @@
 #!/usr/bin/env python
-"""bench.py - the hot path's benchmark (contract in the task prompt, section 4).
+"""bench.py - the hot path's benchmark.
 
     python bench.py --gpus 1 --steps K --warmup W            # B200 arm
     python bench.py --impl reference --steps K --warmup W    # reference CPU arm
     torchrun --nproc-per-node N ... bench.py --gpus N ...    # MCU-row sharded, weak scaling
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's result
+
+--dump-outputs DIR writes DIR/ret.npy (the call's return code) and DIR/coef<k>.npy: a fixed, seeded
+sample of a quarter of component k's smoothed 8x8 blocks (float32, shape (blocks, 64); exact for the
+int16 coefficients).  The input is the same seeded image in every run, so two builds (or the two arms)
+can be compared array for array.  Ranks of a sharded run prefix their files with rank<r>_.  The reference
+arm's AVX-512 build is called with JPEGQS_TRANSCODE and so returns re-quantized coefficients; the B200
+arm and the reference arm's C port return de-quantized ones.
 
 A "step" is one complete do_quantsmooth pass (all components, all iterations) over one
 synthetic image.  N=1 workload: BASELINE.json's metric configuration, 7680x4320 YCbCr
@@ -30,6 +38,18 @@ sys.path.insert(0, ROOT)
 METRIC = "Mpixels/sec at q=3 niter=3 (8K 4:2:0); achieved HBM GB/s vs peak"
 WIDTH, HEIGHT, SUBSAMPLING, FLAGS, NITER, QUALITY, SEED = 7680, 4320, "420", 0, 3, 50, 12345
 ALGO_BYTES_PER_BLOCK_ITER = 256          # SURVEY.md 8d: 128 B coefficient read + 128 B write
+DUMP_SHARE = 4                           # --dump-outputs keeps 1 block in DUMP_SHARE: 50 MB at 8K 4:2:0
+
+
+def dump_outputs(d, ret, coefs, prefix="", world=1):
+    """ret and a seeded sample of whole blocks of each component's coefficients, as float32 .npy."""
+    os.makedirs(d, exist_ok=True)
+    rng = np.random.RandomState(SEED)
+    np.save(os.path.join(d, prefix + "ret.npy"), np.array([ret], dtype=np.float64))
+    for k, c in enumerate(coefs):
+        blocks = np.asarray(c).reshape(-1, 64)
+        keep = np.sort(rng.choice(len(blocks), len(blocks) // (DUMP_SHARE * world), replace=False))
+        np.save(os.path.join(d, f"{prefix}coef{k}.npy"), blocks[keep].astype(np.float32))
 
 
 def peaks():
@@ -152,6 +172,7 @@ def run_reference_arm(args, rank, world):
     ol.ensure_built()
     kind = "reference" if ol.have_ref("avx512") else "port"
     times = []
+    result = None
     cores = None
     nthreads = 0
     if kind == "reference":
@@ -174,17 +195,19 @@ def run_reference_arm(args, rank, world):
             lib = ol.reflib("avx512")
             cores = nthreads
             lib.qsref_take_log()
-            ol.run_reference(im, FLAGS | (8 << 16), NITER, variant="avx512", threads=nthreads)
+            result = ol.run_reference(im, FLAGS | (8 << 16), NITER, variant="avx512", threads=nthreads)
             log = lib.qsref_take_log().decode()
             ms = [float(l.split(":")[1].replace("ms", "")) for l in log.splitlines() if l.startswith("quantsmooth:")]
             dt = ms[-1] / 1e3
         else:
             cores = ol.oraclelib().qso_num_procs()
             t = time.perf_counter()
-            ol.run_oracle(im, FLAGS, NITER, threads=0)
+            result = ol.run_oracle(im, FLAGS, NITER, threads=0)
             dt = time.perf_counter() - t
         if i >= args.warmup:
             times.append(dt)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, result[0], [c.coef for c in result[1].comps])
     total = sum(times)
     mpix = WIDTH * HEIGHT / 1e6
     value = mpix * len(times) / total
@@ -211,7 +234,10 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's result as .npy files")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -297,7 +323,7 @@ def main():
     sampler.t0 = time.perf_counter()
     e0.record()
     for i in range(K):
-        step(Wm + i)
+        ret = step(Wm + i)
         launches += ctx.last_launches
         a, b, c, d = ctx.kernel_stats()
         idct_ms += a; idct_n += b; smooth_ms += c; smooth_n += d
@@ -441,6 +467,10 @@ def main():
         sec, kind, cores, how = cpu_reference_time(im, threads=0, runs=5)
         cpu = {"value": round(WIDTH * HEIGHT / 1e6 / sec, 3), "unit": "Mpixels/s", "cores": cores, "kind": kind,
                "sample": f"the full 8K image, 1 warm-up + median of 5 runs ({how})"}
+
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, ret, [t.cpu().numpy() for t in dev_bufs[Wm + K - 1]],
+                     prefix="" if world == 1 else f"rank{rank}_", world=world)
 
     if rank == 0:
         out = {

@@ -1,4 +1,9 @@
-"""Load/save golden cases and build the adversarial inputs used by the edge-case tests."""
+"""Load/save golden cases, look up the reference's stored outputs, and build the adversarial
+inputs used by the edge-case tests."""
+import hashlib
+import json
+import os
+
 import numpy as np
 
 from jpegqs_b200.image import CoefImage, Component, JCS_GRAYSCALE, JCS_YCbCr
@@ -27,6 +32,43 @@ def load_case(path):
     im = CoefImage(int(z["width"]), int(z["height"]), int(z["colorspace"]), comps_in)
     out = CoefImage(int(z["width"]), int(z["height"]), int(z["colorspace"]), comps_out)
     return im, out, int(z["flags"]), int(z["niter"]), int(z["ret"])
+
+
+REFERENCE_OUTPUTS = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_outputs.json")
+_reference_outputs = None
+
+
+def reference_output(key):
+    """What the unmodified reference gave for one test case: written by
+    tests/golden/make_reference_outputs.py, outputs as SHA-256 digests (see the digest helpers)."""
+    global _reference_outputs
+    if _reference_outputs is None:
+        with open(REFERENCE_OUTPUTS) as f:
+            _reference_outputs = json.load(f)
+    return _reference_outputs[key]
+
+
+def digest(*chunks):
+    h = hashlib.sha256()
+    for c in chunks:
+        h.update(c if isinstance(c, bytes) else np.ascontiguousarray(c).tobytes())
+    return h.hexdigest()
+
+
+def file_digest(path):
+    with open(path, "rb") as f:
+        return digest(f.read())
+
+
+def image_digest(ret, image):
+    """Everything oracle_lib.images_equal compares, plus the return code."""
+    parts = [np.array([ret, len(image.comps)], dtype=np.int64)]
+    for c in image.comps:
+        parts += [np.array(c.coef.shape + (c.h_samp, c.v_samp, c.quant is not None), dtype=np.int64),
+                  np.ascontiguousarray(c.coef, dtype=np.int16)]
+        if c.quant is not None:
+            parts.append(np.asarray(c.quant, dtype=np.uint16))
+    return digest(*parts)
 
 
 def _checker_coefs(lo, hi, q):

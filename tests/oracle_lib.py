@@ -1,6 +1,6 @@
 """ctypes bindings for the TEST INFRASTRUCTURE under oracle/:
-  - oracle/_ref/libqsref_{scalar,avx512}.so : the unmodified reference (built here from
-    /root/reference; travels prebuilt to the GPU box)
+  - oracle/_ref/libqsref_{scalar,avx512}.so : the unmodified reference (built by build() through
+    oracle/Makefile where the reference's sources are present)
   - oracle/libqs_oracle.so                  : the C restatement
   - oracle/libfakejpeg.so                   : fake libjpeg front end used to drive any
     do_quantsmooth-shaped function through the libjpeg-facing boundary.
@@ -23,8 +23,8 @@ def ensure_built():
     src = [os.path.join(ORACLE, "qs_oracle.c"), os.path.join(ORACLE, "fakejpeg.c")]
     stale = any((not os.path.exists(n)) or os.path.getmtime(n) < os.path.getmtime(s)
                 for n, s in zip(need, src))
-    if stale or (os.path.exists("/root/reference/quantsmooth.h") and not have_ref()):
-        subprocess.run(["make", "-C", ORACLE, "all"], check=True, capture_output=True)
+    if stale:
+        subprocess.run(["make", "-C", ORACLE, "restatement", "fake"], check=True, capture_output=True)
 
 
 def have_ref(variant="scalar"):

@@ -3,12 +3,15 @@
 CUDA back end) on baseline / progressive / sub-sampled / restart-marker / grayscale files
 written by Pillow's libjpeg-turbo, and markers are copied per `-c`.  GPU leg: the CUDA-backed
 tool must write byte-identical files to oracle/_ref/jpegqs_ref (the same front end linked
-against the UNMODIFIED reference do_quantsmooth, built by oracle/Makefile)."""
+against the UNMODIFIED reference do_quantsmooth, built by oracle/Makefile); the digests of that
+tool's files are stored in tests/golden/reference_outputs.json (see reference_outputs())."""
 import os
 import subprocess
 
 import numpy as np
 import pytest
+
+from golden_io import file_digest, reference_output
 
 PIL = pytest.importorskip("PIL.Image")
 
@@ -45,15 +48,24 @@ FILES = [
 ]
 
 
-@pytest.fixture(scope="module")
-def jpegs(tmp_path_factory):
-    d = tmp_path_factory.mktemp("jpegs")
+def make_jpegs(d):
     out = {}
     for k, (name, w, h, gray, kw) in enumerate(FILES):
-        p = str(d / (name + ".jpg"))
+        p = os.path.join(d, name + ".jpg")
         _picture(w, h, gray, k).save(p, comment=b"made by the test suite", **kw)
         out[name] = p
     return out
+
+
+@pytest.fixture(scope="module")
+def jpegs(tmp_path_factory):
+    return make_jpegs(str(tmp_path_factory.mktemp("jpegs")))
+
+
+def check_input(name, path):
+    """The stored outputs of the reference were made from these very files."""
+    assert file_digest(path) == reference_output(f"input/{name}"), \
+        f"{name}: this Pillow writes other bytes than the one the reference outputs were made with"
 
 
 def _pixels(path):
@@ -277,24 +289,25 @@ def test_no_cpu_fallback_in_the_tool(jpegs, tmp_path):
     assert not out.exists()
 
 
-@pytest.mark.gpu
-@pytest.mark.skipif(not os.path.exists(REF_EXE), reason="oracle/_ref/jpegqs_ref not built")
-@pytest.mark.parametrize("name,args", [
+REF_TOOL_CASES = [
     ("base420", ["-q", "3"]), ("base420", ["-q", "6", "-n", "2"]), ("prog420", ["-q", "4", "-n", "2", "-o"]),
     ("base444", ["-q", "5", "-n", "2"]), ("gray", ["-q", "3", "-n", "4"]), ("opt422", ["-q", "6"]),
     ("prog444", ["-q", "1", "-n", "2"]), ("rst", ["-q", "0"]), ("progrst", ["-q", "1", "-o"]),
     ("opt422", ["-q", "2", "-o"]),
     ("tinyprog", ["-q", "3"]), ("base420", ["-f", "16", "-n", "2"]),
-])
+]
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("name,args", REF_TOOL_CASES)
 def test_cuda_tool_writes_the_reference_tools_bytes(jpegs, tmp_path, name, args):
     # UPSAMPLE_UV cases use widths that are multiples of the MCU: for other widths the reference
     # reads uninitialised memory when it pads the up-sampled plane (DESIGN.md "reference quirks")
-    a, b = str(tmp_path / "cuda.jpg"), str(tmp_path / "ref.jpg")
+    check_input(name, jpegs[name])
+    a = str(tmp_path / "cuda.jpg")
     r1 = subprocess.run([EXE, "-i", "0"] + args + [jpegs[name], a], capture_output=True, text=True)
-    r2 = subprocess.run([REF_EXE, "-i", "0"] + args + [jpegs[name], b], capture_output=True, text=True)
     assert r1.returncode == 0, r1.stderr
-    assert r2.returncode == 0, r2.stderr
-    assert open(a, "rb").read() == open(b, "rb").read()
+    assert file_digest(a) == reference_output(f"jpegqs_ref/{name} {' '.join(args)}")
     PIL.open(a).load()                      # and it is a decodable JPEG
 
 
@@ -388,3 +401,14 @@ def test_codec_survives_corrupt_input(jpegs, tmp_path):
         r2 = subprocess.run([exe, "-n", "0", "-i", "0", str(f), str(out)], capture_output=True, timeout=60, env=env)
         assert r2.returncode == r.returncode, (it, r.returncode, r2.returncode, r2.stderr.decode()[-800:])
         assert (out.read_bytes() if out.exists() else None) == want, it
+
+
+def reference_outputs(tmpdir):
+    """The inputs' digests and oracle/_ref/jpegqs_ref's files for the cases above."""
+    jpegs = make_jpegs(tmpdir)
+    out = {f"input/{name}": file_digest(p) for name, p in jpegs.items()}
+    for name, args in REF_TOOL_CASES:
+        b = os.path.join(tmpdir, "ref.jpg")
+        subprocess.run([REF_EXE, "-i", "0"] + args + [jpegs[name], b], check=True, capture_output=True)
+        out[f"jpegqs_ref/{name} {' '.join(args)}"] = file_digest(b)
+    return out

@@ -8,7 +8,7 @@ import pytest
 
 import jpegqs_b200 as qs
 import oracle_lib as ol
-from golden_io import adversarial_image
+from golden_io import adversarial_image, image_digest, reference_output
 from jpegqs_b200 import multigpu as mg
 
 pytestmark = pytest.mark.gpu
@@ -85,18 +85,26 @@ def test_progress_sequence_and_cancel(ctx):
     assert ol.images_equal(o1, o2)
 
 
-@pytest.mark.parametrize("flags,niter,ss", [(0, 3, "420"), (7, 2, "420"), (3, 2, "444"), (1, 1, "gray")])
+BOUNDARY_CASES = [(0, 3, "420"), (7, 2, "420"), (3, 2, "444"), (1, 1, "gray")]
+
+
+@pytest.mark.parametrize("flags,niter,ss", BOUNDARY_CASES)
 def test_libjpeg_facing_entry_point(flags, niter, ss):
     """do_quantsmooth(j_decompress_ptr, jvirt_barray_ptr*, jpegqs_control_t*) through the
-    fake libjpeg front end, rows scattered in memory like libjpeg's virtual arrays."""
+    fake libjpeg front end, rows scattered in memory like libjpeg's virtual arrays; the
+    reference's result through the same front end is stored (reference_outputs())."""
     lib = qs.cuda.load()
     im = qs.synth.make_image(120, 72, ss)
     ret, out = ol.run_libjpeg_boundary(lib.do_quantsmooth, im, flags | 64, niter, scatter_rows=True)
     oret, oout = ol.run_oracle(im, flags, niter)
     assert ret == oret and ol.images_equal(out, oout)
-    if ol.have_ref("scalar"):
-        rret, rout = ol.run_reference(im, flags, niter, scatter_rows=True)
-        assert ret == rret and ol.images_equal(out, rout)
+    assert image_digest(ret, out) == reference_output(f"libjpeg_boundary/{flags},{niter},{ss}")
+
+
+def reference_outputs(tmpdir):
+    return {f"libjpeg_boundary/{flags},{niter},{ss}":
+            image_digest(*ol.run_reference(qs.synth.make_image(120, 72, ss), flags, niter, scatter_rows=True))
+            for flags, niter, ss in BOUNDARY_CASES}
 
 
 def test_batch_entry_point(ctx):

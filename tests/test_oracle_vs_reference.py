@@ -1,17 +1,14 @@
 """Pins the C restatement (oracle/qs_oracle.c) against the UNMODIFIED reference
-(oracle/_ref/libqsref_scalar.so, the -DNO_SIMD build of /root/reference/quantsmooth.h).
-Skipped where oracle/_ref is absent; the committed golden vectors (test_golden.py) cover
-that case."""
-import ctypes as C
-
+(oracle/_ref/libqsref_scalar.so, the -DNO_SIMD build of the reference's quantsmooth.h).
+What the reference gives for every case below is stored in tests/golden/reference_outputs.json
+(reference_outputs() computes it; tests/golden/make_reference_outputs.py writes it), so the
+tests need no reference build."""
 import numpy as np
 import pytest
 
 import jpegqs_b200 as qs
 import oracle_lib as ol
-from golden_io import adversarial_image
-
-pytestmark = pytest.mark.skipif(not ol.have_ref("scalar"), reason="oracle/_ref not built (needs /root/reference)")
+from golden_io import adversarial_image, digest, image_digest, reference_output
 
 
 def test_natural_order_and_refresh_points():
@@ -30,39 +27,54 @@ def test_natural_order_and_refresh_points():
     assert got == refresh
 
 
-def test_idct_islow_exact():
-    ref, orc = ol.reflib(), ol.oraclelib()
+def _idct_islow(idct):
+    """Digests of the pixels idct makes of 200 random blocks, one per coefficient scale."""
     rng = np.random.RandomState(1)
+    out = []
     for scale in (8, 200, 2047):
+        pixels = []
         for _ in range(200):
             c = rng.randint(-scale, scale + 1, size=64).astype(np.int16)
             if rng.rand() < 0.3:
                 c[rng.rand(64) < 0.8] = 0
-            a = np.zeros((8, 24), dtype=np.uint8); b = np.zeros((8, 24), dtype=np.uint8)
-            ref.qsref_idct_islow(c.ctypes.data, a.ctypes.data, 24)
-            orc.qso_idct_islow(c.ctypes.data, b.ctypes.data, 24)
-            assert np.array_equal(a, b)
+            a = np.zeros((8, 24), dtype=np.uint8)
+            idct(c.ctypes.data, a.ctypes.data, 24)
+            pixels.append(a)
+        out.append(digest(*pixels))
+    return out
+
+
+def test_idct_islow_exact():
+    assert _idct_islow(ol.oraclelib().qso_idct_islow) == reference_output("idct_islow")
+
+
+def _float_dct(fn):
+    rng = np.random.RandomState(2)
+    out = []
+    for _ in range(300):
+        x = (rng.rand(64).astype(np.float32) - 0.5) * np.float32(rng.choice([1, 255, 4096]))
+        a = np.zeros(64, dtype=np.float32)
+        fn(x.copy().ctypes.data, a.ctypes.data)
+        out.append(a.view(np.uint32))
+    return digest(*out)
 
 
 def test_float_dcts_bit_exact():
-    ref, orc = ol.reflib(), ol.oraclelib()
-    rng = np.random.RandomState(2)
-    for _ in range(300):
-        x = (rng.rand(64).astype(np.float32) - 0.5) * np.float32(rng.choice([1, 255, 4096]))
-        for fr, fo in ((ref.qsref_fdct_float, orc.qso_fdct_float), (ref.qsref_idct_float, orc.qso_idct_float)):
-            a = np.zeros(64, dtype=np.float32); b = np.zeros(64, dtype=np.float32)
-            xa, xb = x.copy(), x.copy()
-            fr(xa.ctypes.data, a.ctypes.data); fo(xb.ctypes.data, b.ctypes.data)
-            assert np.array_equal(a.view(np.uint32), b.view(np.uint32))
+    orc = ol.oraclelib()
+    assert _float_dct(orc.qso_fdct_float) == reference_output("fdct_float")
+    assert _float_dct(orc.qso_idct_float) == reference_output("idct_float")
+
+
+def _tables(fn, flags):
+    a = np.zeros((64, 272 if flags else 160), dtype=np.float32)
+    fn(flags, a.ctypes.data)
+    return digest(a.view(np.uint32))
 
 
 @pytest.mark.parametrize("flags", [0, 1])
 def test_tables_bit_exact(flags):
-    size = 272 if flags else 160
-    a = np.zeros((64, size), dtype=np.float32); b = np.zeros((64, size), dtype=np.float32)
-    assert ol.reflib().qsref_tables(flags, a.ctypes.data) == size
-    ol.oraclelib().qso_tables(flags, b.ctypes.data)
-    assert np.array_equal(a.view(np.uint32), b.view(np.uint32))
+    assert ol.oraclelib().qso_table_size(flags) == (272 if flags else 160)
+    assert _tables(ol.oraclelib().qso_tables, flags) == reference_output(f"tables/{flags}")
 
 
 def test_orig_coef_exhaustive_vs_reference_formula():
@@ -92,21 +104,17 @@ CASES = [
 @pytest.mark.parametrize("w,h,ss,flags,niter,quality", CASES)
 def test_driver_matches_reference(w, h, ss, flags, niter, quality):
     im = qs.synth.make_image(w, h, ss, quality=quality)
-    r1, o1 = ol.run_reference(im, flags, niter)
-    r2, o2 = ol.run_oracle(im, flags, niter)
-    assert r1 == r2
-    assert ol.diff_count(o1, o2) == 0 and ol.images_equal(o1, o2)
+    assert image_digest(*ol.run_oracle(im, flags, niter)) == reference_output(f"driver/{w},{h},{ss},{flags},{niter},{quality}")
 
 
-@pytest.mark.parametrize("kind,flags,niter", [("nan", 0, 1), ("badcoef", 0, 2), ("bigquant", 0, 2),
-                                              ("zeroquant", 0, 2), ("flat", 1, 2), ("q1", 0, 3),
-                                              ("badcoef", 7, 2), ("bigquant", 7, 1)])
+ADVERSARIAL = [("nan", 0, 1), ("badcoef", 0, 2), ("bigquant", 0, 2), ("zeroquant", 0, 2), ("flat", 1, 2), ("q1", 0, 3),
+               ("badcoef", 7, 2), ("bigquant", 7, 1)]
+
+
+@pytest.mark.parametrize("kind,flags,niter", ADVERSARIAL)
 def test_adversarial_matches_reference(kind, flags, niter):
     im = adversarial_image(kind)
-    r1, o1 = ol.run_reference(im, flags, niter)
-    r2, o2 = ol.run_oracle(im, flags, niter)
-    assert r1 == r2
-    assert ol.images_equal(o1, o2)
+    assert image_digest(*ol.run_oracle(im, flags, niter)) == reference_output(f"adversarial/{kind},{flags},{niter}")
 
 
 def test_nan_case_moves_coefficients():
@@ -119,31 +127,33 @@ def test_nan_case_moves_coefficients():
 
 
 def test_non_contiguous_rows_and_threads():
+    """The reference's result with scattered rows and 3 threads (stored) is the restatement's
+    with 1 and with 3 threads."""
     im = qs.synth.make_image(96, 80, "420")
-    _, a = ol.run_reference(im, 7, 2, scatter_rows=True, threads=3)
-    _, b = ol.run_reference(im, 7, 2, threads=1)
-    assert ol.images_equal(a, b)
+    want = reference_output("scattered_rows_3_threads")
+    for threads in (1, 3):
+        assert image_digest(*ol.run_oracle(im, 7, 2, threads=threads)) == want
+
+
+def _progress(run):
+    """The progress sequence of a full run, then a run cancelled at the second callback."""
+    im = qs.synth.make_image(96, 80, "420")
+    seq = []
+    run(im, 0, 3, progprec=7, progress=lambda d, cur, mx: seq.append([cur, mx]) or 0)
+    cancelled = []
+    ret, out = run(im, 0, 3, progprec=7,
+                   progress=lambda d, cur, mx: (cancelled.append(cur), 5 if len(cancelled) >= 2 else 0)[1])
+    return {"sequence": seq, "cancelled": cancelled, "cancelled_ret": ret, "cancelled_result": image_digest(ret, out)}
 
 
 def test_progress_sequence_and_cancel():
-    im = qs.synth.make_image(96, 80, "420")
-    seq_ref, seq_orc = [], []
-    ol.run_reference(im, 0, 3, progprec=7, progress=lambda d, cur, mx: seq_ref.append((cur, mx)) or 0)
-    ol.run_oracle(im, 0, 3, progprec=7, progress=lambda d, cur, mx: seq_orc.append((cur, mx)) or 0)
-    assert seq_ref == seq_orc and len(seq_ref) > 2
-    # cancel at the second callback
-    def mk(seq):
-        return lambda d, cur, mx: (seq.append(cur), 5 if len(seq) >= 2 else 0)[1]
-    s1, s2 = [], []
-    r1, o1 = ol.run_reference(im, 0, 3, progprec=7, progress=mk(s1))
-    r2, o2 = ol.run_oracle(im, 0, 3, progprec=7, progress=mk(s2))
-    assert r1 == r2 == 5 and s1 == s2
-    assert ol.images_equal(o1, o2)
+    want = reference_output("progress")
+    assert len(want["sequence"]) > 2 and want["cancelled_ret"] == 5
+    assert _progress(ol.run_oracle) == want
 
 
-def test_randomized_sweep_matches_reference():
-    """The same seeded sweep the GPU parity test runs (tests/test_gpu_parity.py), here pinning
-    the checker itself against the unmodified reference."""
+def _sweep():
+    """The same seeded sweep the GPU parity test runs (tests/test_gpu_parity.py)."""
     rng = np.random.RandomState(20260923)
     modes = ["gray", "444", "422", "420", "440"]
     for case in range(48):
@@ -155,6 +165,31 @@ def test_randomized_sweep_matches_reference():
             w = max(16, w // 16 * 16)
         niter = int(rng.randint(1, 4))
         im = qs.synth.make_image(w, h, ss, quality=quality, seed=1000 + case, noise=int(rng.randint(0, 12)))
-        r1, o1 = ol.run_reference(im, flags, niter)
-        r2, o2 = ol.run_oracle(im, flags, niter)
-        assert r1 == r2 and ol.images_equal(o1, o2), (case, w, h, ss, quality, flags, niter)
+        yield (case, w, h, ss, quality, flags, niter), im
+
+
+def test_randomized_sweep_matches_reference():
+    """The sweep, here pinning the checker itself against the unmodified reference."""
+    want = reference_output("sweep")
+    for (case, w, h, ss, quality, flags, niter), im in _sweep():
+        assert image_digest(*ol.run_oracle(im, flags, niter)) == want[case], (case, w, h, ss, quality, flags, niter)
+
+
+def reference_outputs(tmpdir):
+    """What the reference gives for every case above, keyed as the tests look it up."""
+    ref = ol.reflib()
+    out = {"idct_islow": _idct_islow(ref.qsref_idct_islow)}
+    out["fdct_float"], out["idct_float"] = _float_dct(ref.qsref_fdct_float), _float_dct(ref.qsref_idct_float)
+    for flags in (0, 1):
+        out[f"tables/{flags}"] = _tables(ref.qsref_tables, flags)
+    for w, h, ss, flags, niter, quality in CASES:
+        im = qs.synth.make_image(w, h, ss, quality=quality)
+        out[f"driver/{w},{h},{ss},{flags},{niter},{quality}"] = image_digest(*ol.run_reference(im, flags, niter))
+    for kind, flags, niter in ADVERSARIAL:
+        out[f"adversarial/{kind},{flags},{niter}"] = image_digest(*ol.run_reference(adversarial_image(kind), flags, niter))
+    im = qs.synth.make_image(96, 80, "420")
+    out["scattered_rows_3_threads"] = image_digest(*ol.run_reference(im, 7, 2, scatter_rows=True, threads=3))
+    assert out["scattered_rows_3_threads"] == image_digest(*ol.run_reference(im, 7, 2, threads=1))
+    out["progress"] = _progress(ol.run_reference)
+    out["sweep"] = [image_digest(*ol.run_reference(im, c[-2], c[-1])) for c, im in _sweep()]
+    return out

@@ -9,8 +9,10 @@ GPU leg: the reference's OWN callers run on the CUDA back end with real libjpeg 
 oracle/_ref/refcli_b200 is the unmodified reference quantsmooth.c whose SIMD dispatcher links
 the tier workers exported by libjpegqs_b200.so; example_b200 is the reference's example.c
 (jpegqs_start_decompress -> jpeg_read_scanlines) - and must reproduce the all-CPU builds of the
-same sources (refcli_cpu / example_cpu) byte for byte."""
+same sources (refcli_cpu / example_cpu) byte for byte.  What the all-CPU builds write is stored in
+tests/golden/reference_outputs.json (see reference_outputs())."""
 import glob
+import json
 import os
 import subprocess
 
@@ -27,25 +29,25 @@ _so = sorted(glob.glob(os.path.join(os.path.dirname(os.path.realpath(_PIL.__file
 JPEG_SO = os.path.realpath(_so[0]) if _so else None
 pytestmark = pytest.mark.skipif(JPEG_SO is None, reason="no libjpeg shared library inside Pillow")
 
-from test_cli import FILES, _picture  # noqa: E402
+from golden_io import digest, file_digest, reference_output  # noqa: E402
+from test_cli import _picture, check_input, make_jpegs  # noqa: E402
 
 
-@pytest.fixture(scope="module")
-def jpegs(tmp_path_factory):
-    d = tmp_path_factory.mktemp("real")
-    out = {}
-    for k, (name, w, h, gray, kw) in enumerate(FILES):
-        p = str(d / (name + ".jpg"))
-        _picture(w, h, gray, k).save(p, comment=b"made by the test suite", **kw)
-        out[name] = p
+def make_real_jpegs(d):
+    out = make_jpegs(d)
     # sizes that are multiples of the MCU: the reference's UPSAMPLE_UV reads uninitialised memory
     # otherwise (DESIGN.md "reference quirks"), so q6 is compared on these only
     for name, w, h, kw in (("mcu420", 192, 144, dict(quality=60)), ("mcuprog", 256, 160, dict(quality=85, progressive=True)),
                            ("mcu422", 160, 96, dict(quality=40, subsampling=1))):
-        p = str(d / (name + ".jpg"))
+        p = os.path.join(d, name + ".jpg")
         _picture(w, h, False, 11).save(p, **kw)
         out[name] = p
     return out
+
+
+@pytest.fixture(scope="module")
+def jpegs(tmp_path_factory):
+    return make_real_jpegs(str(tmp_path_factory.mktemp("real")))
 
 
 DUMP = r'''
@@ -108,64 +110,110 @@ def _have(*names):
     return all(os.path.exists(os.path.join(REFDIR, n)) for n in names)
 
 
-@pytest.mark.skipif(not _have("refcli_cpu", "jpegqs_ref"), reason="oracle/_ref not built")
+def _b200_env():
+    """refcli_b200 / example_b200 load libjpegqs_b200.so from this tree's csrc/, named explicitly:
+    their run path only finds it while oracle/_ref sits inside the tree it was built in."""
+    path = os.environ.get("LD_LIBRARY_PATH")
+    return dict(os.environ, LD_LIBRARY_PATH=CSRC + (os.pathsep + path if path else ""))
+
+
+REFCLI_CASES = [(name, args) for name in ("base420", "gray", "prog420", "opt422", "rst")
+                for args in (["-q", "3", "-n", "2"], ["-q", "4", "-n", "1", "-o"], ["-q", "2"])]
+
+
+@pytest.mark.skipif(not _have("jpegqs_ref"), reason="oracle/_ref not built")
 def test_reference_cli_on_real_libjpeg_writes_this_codecs_bytes(jpegs, tmp_path):
-    """quantsmooth.c + libjpeg-turbo vs the same smoothing behind csrc/jpegcoef.c + jpegqs.c:
-    the files are byte-identical, i.e. the codec reproduces jpeg_copy_critical_parameters +
-    jpeg_write_coefficients + jcopy_markers (JFIF / Adobe handling included)."""
-    for name in ("base420", "gray", "prog420", "opt422", "rst"):
-        for args in (["-q", "3", "-n", "2"], ["-q", "4", "-n", "1", "-o"], ["-q", "2"]):
-            a, b = str(tmp_path / "real.jpg"), str(tmp_path / "jq.jpg")
-            r1 = subprocess.run([os.path.join(REFDIR, "refcli_cpu"), "-i", "0"] + args + [jpegs[name], a], capture_output=True)
-            r2 = subprocess.run([os.path.join(REFDIR, "jpegqs_ref"), "-i", "0"] + args + [jpegs[name], b], capture_output=True)
-            assert r1.returncode == 0 and r2.returncode == 0
-            assert open(a, "rb").read() == open(b, "rb").read(), (name, args)
+    """quantsmooth.c + libjpeg-turbo (refcli_cpu, stored) vs the same smoothing behind
+    csrc/jpegcoef.c + jpegqs.c: the files are byte-identical, i.e. the codec reproduces
+    jpeg_copy_critical_parameters + jpeg_write_coefficients + jcopy_markers (JFIF / Adobe handling
+    included)."""
+    for name, args in REFCLI_CASES:
+        check_input(name, jpegs[name])
+        b = str(tmp_path / "jq.jpg")
+        r2 = subprocess.run([os.path.join(REFDIR, "jpegqs_ref"), "-i", "0"] + args + [jpegs[name], b], capture_output=True)
+        assert r2.returncode == 0
+        assert file_digest(b) == reference_output(f"refcli_cpu/{name} {' '.join(args)}"), (name, args)
 
 
-@pytest.mark.skipif(not _have("refcli_cpu"), reason="oracle/_ref not built")
 def test_random_files_one_thread_threaded_and_libjpeg_turbo_agree(tmp_path):
     """A short run of tools/codec_difftest.py: random size / quality / sub-sampling / optimised tables /
-    restart intervals / progressive files; the lossless transcode must give libjpeg-turbo's bytes with the
-    one-thread reader and with the threaded reader (random thread count and chunk size)."""
-    r = subprocess.run([os.sys.executable, os.path.join(ROOT, "tools", "codec_difftest.py"), "77", "30"], cwd=str(tmp_path),
-                       capture_output=True, text=True, timeout=900)
+    restart intervals / progressive files; the lossless transcode must give libjpeg-turbo's bytes (as
+    refcli_cpu wrote them, stored) with the one-thread reader and with the threaded reader (random thread
+    count and chunk size)."""
+    digests = tmp_path / "refcli_cpu.json"
+    digests.write_text(json.dumps(reference_output("codec_difftest/77 30")))
+    r = subprocess.run([os.sys.executable, os.path.join(ROOT, "tools", "codec_difftest.py"), "77", "30", str(digests)],
+                       cwd=str(tmp_path), capture_output=True, text=True, timeout=900)
     assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
     assert "done 30 bad 0" in r.stdout, r.stdout[-2000:]
 
 
+B200_CLI_CASES = {"-q 3": ("base420", "prog420", "gray", "rst"), "-q 4 -n 2": ("prog420", "opt422", "base444"),
+                  "-q 5 -n 2": ("base420", "mcu420", "base444"), "-q 6": ("mcu420", "mcuprog", "mcu422"),
+                  "-q 1": ("gray", "opt422", "rst"), "-q 3 -o": ("base420", "prog420", "opt422")}
+
+
 @pytest.mark.gpu
-@pytest.mark.skipif(not _have("refcli_cpu", "refcli_b200"), reason="oracle/_ref not built")
+@pytest.mark.skipif(not _have("refcli_b200"), reason="oracle/_ref not built")
 @pytest.mark.parametrize("args", [["-q", "3"], ["-q", "4", "-n", "2"], ["-q", "5", "-n", "2"], ["-q", "6"], ["-q", "1"], ["-q", "3", "-o"]])
 def test_unmodified_reference_cli_runs_on_the_cuda_back_end(jpegs, tmp_path, args):
     # each file costs a fresh process with its CUDA start-up: the flavours are spread over the argument sets
     # (q6 on MCU-multiple sizes only, see the fixture)
-    names = {"-q 3": ("base420", "prog420", "gray", "rst"), "-q 4 -n 2": ("prog420", "opt422", "base444"),
-             "-q 5 -n 2": ("base420", "mcu420", "base444"), "-q 6": ("mcu420", "mcuprog", "mcu422"),
-             "-q 1": ("gray", "opt422", "rst"), "-q 3 -o": ("base420", "prog420", "opt422")}[" ".join(args)]
-    for name in names:
-        a, b = str(tmp_path / "cpu.jpg"), str(tmp_path / "b200.jpg")
-        r1 = subprocess.run([os.path.join(REFDIR, "refcli_cpu"), "-i", "0"] + args + [jpegs[name], a], capture_output=True, text=True)
-        r2 = subprocess.run([os.path.join(REFDIR, "refcli_b200"), "-i", "16"] + args + [jpegs[name], b], capture_output=True, text=True)
-        assert r1.returncode == 0 and r2.returncode == 0, (r1.stderr, r2.stderr)
+    for name in B200_CLI_CASES[" ".join(args)]:
+        check_input(name, jpegs[name])
+        b = str(tmp_path / "b200.jpg")
+        r2 = subprocess.run([os.path.join(REFDIR, "refcli_b200"), "-i", "16"] + args + [jpegs[name], b],
+                            capture_output=True, text=True, env=_b200_env())
+        assert r2.returncode == 0, r2.stderr
         assert "CUDA sm_100a" in r2.stderr, r2.stderr            # it really went through the tier slot into the GPU
-        assert open(a, "rb").read() == open(b, "rb").read(), (name, args)
+        assert file_digest(b) == reference_output(f"refcli_cpu/{name} {' '.join(args)}"), (name, args)
+
+
+def _rgb_digest(path):
+    a = np.asarray(PIL.open(path).convert("RGB"))
+    return digest(np.array(a.shape), a)
+
+
+EXAMPLE_FILES = ("mcu420", "mcuprog", "mcu422", "gray", "base444")
 
 
 @pytest.mark.gpu
-@pytest.mark.skipif(not _have("example_cpu", "example_b200"), reason="oracle/_ref not built")
+@pytest.mark.skipif(not _have("example_b200"), reason="oracle/_ref not built")
 def test_reference_example_decodes_through_the_helpers_on_the_cuda_back_end(jpegs, tmp_path):
     """example.c: jpeg_read_header -> jpegqs_start_decompress (q6, n3, progress callback) ->
     jpeg_read_scanlines -> jpegqs_finish_decompress -> BMP, with real libjpeg doing the IDCT /
     colour conversion after the re-armed decoder (quantsmooth.h:2861-2876).  Same pixels, same
-    progress lines as the all-CPU build; and the device renderer (jpegqs --ppm) gives them too."""
+    progress lines as the all-CPU build (example_cpu, stored); and the device renderer
+    (jpegqs --ppm) gives them too."""
     exe = os.path.join(CSRC, "jpegqs")
-    for name in ("mcu420", "mcuprog", "mcu422", "gray", "base444"):
-        a, b = str(tmp_path / "cpu.bmp"), str(tmp_path / "b200.bmp")
-        r1 = subprocess.run([os.path.join(REFDIR, "example_cpu"), jpegs[name], a], capture_output=True, text=True)
-        r2 = subprocess.run([os.path.join(REFDIR, "example_b200"), jpegs[name], b], capture_output=True, text=True)
-        assert r1.returncode == 0 and r2.returncode == 0, (r1.stderr, r2.stderr)
-        assert r1.stdout == r2.stdout, name                       # the progress callback sequence
-        assert open(a, "rb").read() == open(b, "rb").read(), name
+    for name in EXAMPLE_FILES:
+        check_input(name, jpegs[name])
+        want = reference_output(f"example_cpu/{name}")
+        b = str(tmp_path / "b200.bmp")
+        r2 = subprocess.run([os.path.join(REFDIR, "example_b200"), jpegs[name], b], capture_output=True, text=True,
+                            env=_b200_env())
+        assert r2.returncode == 0, r2.stderr
+        assert r2.stdout == want["stdout"], name                  # the progress callback sequence
+        assert file_digest(b) == want["bmp"], name
         ppm = str(tmp_path / "dev.ppm")
         assert subprocess.run([exe, "-q", "6", "-i", "0", "--ppm", jpegs[name], ppm]).returncode == 0
-        assert np.array_equal(np.asarray(PIL.open(ppm).convert("RGB")), np.asarray(PIL.open(a).convert("RGB"))), name
+        assert _rgb_digest(ppm) == want["rgb"], name
+
+
+def reference_outputs(tmpdir):
+    """The inputs' digests and what refcli_cpu and example_cpu write for the cases above."""
+    jpegs = make_real_jpegs(tmpdir)
+    out = {f"input/{name}": file_digest(p) for name, p in jpegs.items()}
+    cases = REFCLI_CASES + [(name, a.split()) for a, names in B200_CLI_CASES.items() for name in names]
+    for name, args in cases:
+        a = os.path.join(tmpdir, "cpu.jpg")
+        subprocess.run([os.path.join(REFDIR, "refcli_cpu"), "-i", "0"] + args + [jpegs[name], a], check=True, capture_output=True)
+        out[f"refcli_cpu/{name} {' '.join(args)}"] = file_digest(a)
+    for name in EXAMPLE_FILES:
+        a = os.path.join(tmpdir, "cpu.bmp")
+        r = subprocess.run([os.path.join(REFDIR, "example_cpu"), jpegs[name], a], check=True, capture_output=True, text=True)
+        out[f"example_cpu/{name}"] = {"stdout": r.stdout, "bmp": file_digest(a), "rgb": _rgb_digest(a)}
+    r = subprocess.run([os.sys.executable, os.path.join(ROOT, "tools", "codec_difftest.py"), "77", "30", "--record"],
+                       cwd=tmpdir, check=True, capture_output=True, text=True)
+    out["codec_difftest/77 30"] = json.loads(r.stdout.splitlines()[-1])
+    return out
