@@ -167,50 +167,11 @@ int jpegqs_cuda_multi_plan(const jpegqs_cuda_multi *m, const jpegqs_cuda_image *
 /* host buffers / block-row tables like jpegqs_cuda_run_host; no progress callback */
 int jpegqs_cuda_run_host_multi(jpegqs_cuda_multi *m, jpegqs_cuda_image *img, int flags, int niter);
 
-/* ---- pass-level entry points (multi-GPU slabs: the caller exchanges halo rows between
- *      the passes; see DESIGN.md section 5).  All pointers are DEVICE pointers. ---------- */
-typedef struct {
-	int16_t *coef;             /* [hblk][wblk][64] of this slab                            */
-	uint8_t *plane;            /* jpegqs_cuda_plane_bytes(wblk, hblk) bytes                */
-	const uint8_t *plane2;     /* down-sampled luma plane of the same geometry, or NULL    */
-	uint32_t wblk, hblk;       /* hblk = block rows held by this slab                      */
-	uint16_t quant[64];        /* raw quantval                                             */
-	int32_t luma;              /* !ci || colour space != YCbCr (quantsmooth.h:2639)        */
-	int32_t top_edge;          /* slab touches the image top / bottom: replicate the       */
-	int32_t bottom_edge;       /* border row there (2618-2619) instead of expecting a halo */
-} jpegqs_cuda_job;
-
+/* ---- geometry of the device's pixel planes -----------------------------------------------
+ * stride = 8*wblk + 2*pad bytes per row; hblk*8 pixel rows plus one halo row above and below */
 size_t jpegqs_cuda_plane_bytes(uint32_t wblk, uint32_t hblk);
 int jpegqs_cuda_plane_stride(uint32_t wblk);
 int jpegqs_cuda_plane_pad(void);   /* byte offset of pixel column 0 inside a plane row */
-
-#define JPEGQS_PASS_DEQUANT 1      /* iteration 0: coef *= quantval, range check (2596-2603) */
-#define JPEGQS_PASS_CLAMP   2      /* write coefficients back clamped to +-1023 (2670-2689)  */
-/* IDCT pass (2589-2620): renders each job's plane (+ replicated borders).  *bad receives a
- * bit mask (bit i = job i, jobs >= 31 share bit 31) of the jobs in which a de-quantized
- * coefficient left [-2048, 2047] (host sync).  bad may be NULL. */
-int jpegqs_cuda_pass_idct(jpegqs_cuda_ctx *ctx, int njobs, const jpegqs_cuda_job *jobs, int mode,
-		int *bad, void *stream);
-/* smoothing pass (2627-2640): quantsmooth_block on every block of every job */
-int jpegqs_cuda_pass_smooth(jpegqs_cuda_ctx *ctx, int njobs, const jpegqs_cuda_job *jobs, int flags,
-		int clamp_out, void *stream);
-
-/* luma -> chroma hand-over for slabs (JOINT_YUV / UPSAMPLE_UV): the down-sampled luma plane
- * of quantsmooth.h:2753-2815 for one slab.  Rows are addressed inside the WHOLE component:
- * y_row0 / c_row0 = first luma / chroma block row of the slab, *_hblk_total = block rows of the
- * whole component.  Writes the slab's rows of plane2 (chroma slab geometry, c_rows block rows)
- * incl. the left/right border and, at an image edge, the replicated border rows; interior
- * halo rows (row -1 / row c_rows*8 of the slab) must be exchanged by the caller. */
-int jpegqs_cuda_pass_downsample(jpegqs_cuda_ctx *ctx, const uint8_t *yplane, uint32_t y_wblk,
-		uint32_t y_row0, uint32_t y_hblk_total, uint8_t *plane2, uint32_t c_wblk, uint32_t c_rows, uint32_t c_row0,
-		uint32_t c_hblk_total, int ws, int hs, int top_edge, int bottom_edge, void *stream);
-/* upsample_row + FDCT (quantsmooth.h:2691-2752) for one chroma component of one slab: fills
- * coef_up [y_rows][y_wblk][64]; scratch = y_wblk*8 * y_rows*8 bytes of device memory.  The
- * chroma plane and plane2 need valid halo rows (3x3 windows). */
-int jpegqs_cuda_pass_upsample(jpegqs_cuda_ctx *ctx, const uint8_t *cplane, const uint8_t *plane2,
-		uint32_t c_wblk, const uint8_t *yplane, uint32_t y_wblk, uint32_t y_rows, uint32_t y_row0,
-		int16_t *coef_up, uint8_t *scratch, int ws, int hs, uint32_t image_width, uint32_t image_height,
-		void *stream);
 
 /* ---- decode to interleaved 8-bit RGB (SURVEY.md 8f row f2) -----------------------------
  * What libjpeg produces after the reference's jpegqs_start_decompress (quantsmooth.h:2880-2904):

@@ -688,16 +688,19 @@ extern "C" void jpegqs_cuda_kernel_stats(const jpegqs_cuda_ctx *ctx, float *idct
 }
 
 /* ------------------------------------------------------------------------------------------
- * whole-image driver
+ * The two drivers, both restating the reference driver do_quantsmooth (quantsmooth.h:2404-2878):
+ * run_images (whole images; the host decides `stop`) and run_slab (one slab of an image sharded
+ * by MCU rows; the device decides `stop`).  Each has its own iteration loop; everything else they
+ * share is below.
  * ------------------------------------------------------------------------------------------ */
 struct CompWork {
 	int img, ci;
 	jpegqs_cuda_comp *c;
 	int16_t *coef_dev; uint8_t *plane;
 	int W, H, luma, qslot;
+	int qval;              /* OR of the raw quant values (2501-2504) */
 	int niter2, extra;
 	bool iterate;          /* takes part in the IDCT / smoothing iterations */
-	bool dequant_only;     /* stop was already set: quantsmooth.h:2551-2566 */
 	bool done_clamp;
 	bool downloaded;       /* the slab pipeline already sent the coefficients back */
 	/* host side (host entry points only): pinned memory the copy engines use, and the block-row
@@ -717,13 +720,292 @@ struct ImgState {
 	int ngroups;
 };
 
+#define QS_MAX_SLABS 16    /* upload / download units of one group of a host entry point */
+
+/* start of a run: counters, niter clamp (quantsmooth.h:2455-2456), and nothing of an earlier
+ * (failed) call may linger in the I/O threads */
+static int run_start(jpegqs_cuda_ctx *ctx, int *niter) {
+	CK(cudaSetDevice(ctx->device));
+	ctx->launches = 0; ctx->last_ms = 0;
+	ctx->ev_kind.clear(); ctx->ev_used = 0;
+	*niter = std::min(std::max(*niter, 0), 100);
+	if (ctx->up) ctx->up->drain();
+	if (ctx->down) ctx->down->drain();
+	ctx->io_ev_used = 0;
+	return 0;
+}
+
+/* start of one image: need_downsample (2447-2453) and the early return of 2458 (s.skip) */
+static int image_start(ImgState &s, jpegqs_cuda_image *im, int flags, int niter) {
+	memset(&s, 0, sizeof(s)); s.im = im; s.stop_ci = 1 << 30;
+	im->upsampled = 0;
+	if (im->ncomp < 1 || im->ncomp > JPEGQS_CUDA_MAX_COMP) return JPEGQS_ERR_ARG;
+	s.need_downsample = (flags & (QS_JOINT_YUV | QS_UPSAMPLE_UV)) && im->is_ycbcr && im->ncomp >= 3 &&
+			im->comp[1].h_samp == 1 && im->comp[1].v_samp == 1 &&
+			im->comp[2].h_samp == 1 && im->comp[2].v_samp == 1;
+	s.skip = niter <= 0 && !((flags & QS_UPSAMPLE_UV) && s.need_downsample);
+	if (!s.skip && s.need_downsample && (im->comp[1].wblk != im->comp[2].wblk || im->comp[1].hblk != im->comp[2].hblk))
+		return JPEGQS_ERR_ARG;
+	return 0;
+}
+
+/* Device arena and pinned staging of a run.  image_layout walks the images twice with the same
+ * code: the first sweep only counts bytes, the second (after reserve) hands out pointers and
+ * prepares the quant constants. */
+struct Layout {
+	jpegqs_cuda_ctx *ctx;
+	bool on_device, carve;
+	size_t bytes, stage_bytes, stage_pos;
+	int nquant;
+	std::vector<QsQuantDev> qhost;
+	std::vector<std::unique_ptr<int16_t *[]> > rowstore;    /* block-row tables made up for flat pageable arrays */
+	Layout(jpegqs_cuda_ctx *c, bool dev) : ctx(c), on_device(dev), carve(false), bytes(0), stage_bytes(0), stage_pos(0), nquant(0) {}
+	void *take(size_t b) {
+		if (carve) return arena_take(ctx, b);
+		bytes += align256(b);
+		return NULL;
+	}
+	int16_t *stage(size_t b) {
+		char *p = carve ? ctx->stage + stage_pos : NULL;
+		(carve ? stage_pos : stage_bytes) += align256(b);
+		return (int16_t *)p;
+	}
+	/* one coefficient array [hblk][wblk][64]: its device copy, and where the copy engines meet its
+	 * host side - a block-row table gathered into staging, the caller's own pinned array, or a
+	 * flat pageable array cut into rows and staged like a table */
+	int16_t *coef(int16_t *host, int16_t *const *rows, uint32_t wblk, uint32_t hblk, int16_t **pin, int16_t *const **prows) {
+		if (on_device) return host;
+		size_t cb = (size_t)wblk * hblk * 128;
+		int16_t *dev = (int16_t *)take(cb);
+		if (rows) { *prows = rows; *pin = stage(cb); }
+		else if (is_pinned(host)) { *prows = NULL; *pin = host; }
+		else {
+			if (carve) {
+				rowstore.emplace_back(new int16_t *[hblk ? hblk : 1]);
+				int16_t **t = rowstore.back().get();
+				for (uint32_t y = 0; y < hblk; y++) t[y] = host + (size_t)y * wblk * 64;
+				*prows = t;
+			}
+			*pin = stage(cb);
+		}
+		return dev;
+	}
+	int quant(const uint16_t *raw, int *val) {
+		if (!carve) { nquant++; return -1; }
+		QsQuantDev q; quant_prepare(raw, &q, val, ctx->tune_maxn, ctx->tune_uni, ctx->tune_merge);
+		qhost.push_back(q);
+		return (int)qhost.size() - 1;
+	}
+	int reserve() {
+		if (arena_reserve(ctx, bytes + 4096)) return JPEGQS_ERR_CUDA;
+		if (quant_reserve(ctx, nquant)) return JPEGQS_ERR_CUDA;
+		if (stage_bytes && stage_reserve(ctx, stage_bytes)) return JPEGQS_ERR_CUDA;
+		qhost.reserve(nquant);
+		carve = true;
+		return 0;
+	}
+};
+
+/* memory of one image: per component its coefficients, plane and quant slot; the down-sampled
+ * luma plane and, for UPSAMPLE_UV, the up-sampled chroma pixels and coefficients */
+static int image_layout(Layout &ly, ImgState &s, std::vector<CompWork> &W, int img, int flags) {
+	jpegqs_cuda_image *im = s.im;
+	W.resize(im->ncomp);
+	for (int ci = 0; ci < im->ncomp; ci++) {
+		jpegqs_cuda_comp *c = &im->comp[ci]; CompWork &w = W[ci];
+		if (!c->coef && !(!ly.on_device && c->rows) && c->wblk && c->hblk) return JPEGQS_ERR_ARG;
+		memset(&w, 0, sizeof(w));
+		w.img = img; w.ci = ci; w.c = c; w.W = c->wblk; w.H = c->hblk;
+		w.luma = !ci || !im->is_ycbcr;                                    /* 2639 */
+		w.coef_dev = ly.coef(c->coef, c->rows, c->wblk, c->hblk, &w.pin, &w.rows);
+		w.plane = (uint8_t *)ly.take(QS_PLANE_BYTES(c->wblk, c->hblk));
+		w.qslot = ly.quant(c->quant, &w.qval);
+	}
+	if (!s.need_downsample || (im->comp[0].h_samp == 1 && im->comp[0].v_samp == 1)) return 0;
+	s.image2_buf = (uint8_t *)ly.take(QS_PLANE_BYTES(im->comp[1].wblk, im->comp[1].hblk));
+	if (flags & QS_UPSAMPLE_UV) for (int j = 0; j < 2; j++) {
+		jpegqs_cuda_comp *c = &im->comp[1 + j]; CompWork &w = W[1 + j];
+		uint32_t W0 = im->comp[0].wblk, H0 = im->comp[0].hblk;
+		if (!c->coef_up && !(!ly.on_device && c->rows_up)) return JPEGQS_ERR_ARG;
+		s.mem_buf[j] = (uint8_t *)ly.take((size_t)W0 * H0 * 64);       /* up-sampled pixel plane */
+		s.coef_up_dev[j] = ly.coef(c->coef_up, c->rows_up, W0, H0, &w.pin_up, &w.rows_up);
+	}
+	return 0;
+}
+
+/* memory of a run: count, reserve, carve; then the quant constants go up */
+static int run_layout(Layout &ly, ImgState *S, std::vector<CompWork> *W, int nimg, int flags, cudaStream_t st) {
+	jpegqs_cuda_ctx *ctx = ly.ctx;
+	for (int sweep = 0; sweep < 2; sweep++) {
+		if (sweep && ly.reserve()) return JPEGQS_ERR_CUDA;
+		for (int n = 0; n < nimg; n++) {
+			if (S[n].skip) continue;
+			int rc = image_layout(ly, S[n], W[n], n, flags);
+			if (rc) return rc;
+		}
+	}
+	assign_sched_slots(ly.qhost.data(), (int)ly.qhost.size());
+	if (!ly.qhost.empty())
+		CK(cudaMemcpyAsync(ctx->quant_dev, ly.qhost.data(), ly.qhost.size() * sizeof(QsQuantDev), cudaMemcpyHostToDevice, st));
+	ctx->jobs_cache[0].clear(); ctx->jobs_cache[1].clear();
+	return 0;
+}
+
+/* grow-only event pools: per group uploaded / finished (sync_ev) and per slab or band (slab_ev) */
+static int group_events(jpegqs_cuda_ctx *ctx, int ngroups) {
+	while ((int)ctx->sync_ev.size() < 2 * ngroups) {
+		cudaEvent_t e; CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming)); ctx->sync_ev.push_back(e);
+	}
+	while ((int)ctx->slab_ev.size() < 2 * ngroups * QS_MAX_SLABS) {
+		cudaEvent_t e; CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming)); ctx->slab_ev.push_back(e);
+	}
+	return 0;
+}
+
+/* block rows [r0, r1) of a component's coefficients / of its up-sampled coefficients (luma geometry) */
+static IoSeg coef_seg(const CompWork &w, int r0, int r1) {
+	IoSeg sg; sg.dev = w.coef_dev; sg.pin = w.pin; sg.rows = w.rows; sg.wblk = w.W; sg.r0 = r0; sg.r1 = r1;
+	return sg;
+}
+static IoSeg up_seg(const ImgState &s, const CompWork &w, int r0, int r1) {
+	IoSeg sg; sg.dev = s.coef_up_dev[w.ci - 1]; sg.pin = w.pin_up; sg.rows = w.rows_up;
+	sg.wblk = s.im->comp[0].wblk; sg.r0 = r0; sg.r1 = r1;
+	return sg;
+}
+
+/* one component's job; top / bottom: it touches the image's top / bottom edge */
+static QsJob make_job(const jpegqs_cuda_ctx *ctx, const CompWork &w, const uint8_t *plane2, int top, int bottom) {
+	QsJob j; memset(&j, 0, sizeof(j));
+	j.coef = w.coef_dev; j.plane = w.plane; j.plane2 = plane2;
+	j.quant = ctx->quant_dev + w.qslot;
+	j.wblk = w.W; j.hblk = w.H; j.stride = QS_PLANE_STRIDE(w.W); j.nblocks = w.W * w.H;
+	j.luma = w.luma; j.top_edge = top; j.bottom_edge = bottom;
+	return j;
+}
+
+/* the down-sampled luma plane a chroma component is predicted from (JOINT_YUV, 2639) */
+static const uint8_t *plane2_of(const ImgState &s, const CompWork &w, int flags) {
+	return (s.image2 && (flags & QS_JOINT_YUV) && w.ci > 0) ? s.image2 : NULL;
+}
+
+/* IDCT pass (2589-2620) over jobs.  stop_aware: the jobs carry their own bad_slot (run_slab) */
+static int launch_idct(jpegqs_cuda_ctx *ctx, std::vector<QsJob> &jobs, int mode, bool stop_aware, cudaStream_t st) {
+	const QsJob *jd; int tiles;
+	if (upload_jobs(ctx, 0, jobs, st, &jd, &tiles, stop_aware)) return JPEGQS_ERR_CUDA;
+	if (prof_begin(ctx, 0, st)) return JPEGQS_ERR_CUDA;
+	CK(qs_launch_idct_pass(jd, (int)jobs.size(), tiles, mode, ctx->flags_dev, st));
+	if (prof_end(ctx, st)) return JPEGQS_ERR_CUDA;
+	ctx->launches++;
+	return 0;
+}
+
+/* smoothing pass (2627-2640) over jobs: LOW_QUALITY, the packed FP32x2 experiment or the
+ * default kernel.  stop_aware: the kernels consult the run's out-of-range flags (run_slab) */
+static int launch_smooth(jpegqs_cuda_ctx *ctx, std::vector<QsJob> &jobs, int flags, int clampv, bool stop_aware,
+		cudaStream_t st) {
+	const QsJob *jd; int tiles;
+	if (upload_jobs(ctx, 1, jobs, st, &jd, &tiles, stop_aware)) return JPEGQS_ERR_CUDA;
+	const int nj = (int)jobs.size();
+	const int *bad = stop_aware ? ctx->flags_dev : NULL;
+	int *tile_counter = ctx->flags_dev + QS_MAX_JOBS;
+	if (prof_begin(ctx, 1, st)) return JPEGQS_ERR_CUDA;
+	if (flags & QS_LOW_QUALITY) CK(qs_launch_lowq(jd, nj, tiles, flags, clampv, bad, st));
+#ifdef QS_EXPERIMENTS
+	else if (ctx->tune_x2 && !bad) CK(qs_launch_smooth_x2(jd, nj, tiles,
+			(flags & QS_DIAGONALS) ? ctx->tab2_diag : ctx->tab2_plain, ctx->nslots2, tile_counter, flags, clampv,
+			ctx->num_sms, ctx->tune_sync, st));
+#endif
+	else CK(qs_launch_smooth(jd, nj, tiles, (flags & QS_DIAGONALS) ? ctx->tab_diag : ctx->tab_plain, tile_counter,
+			flags, clampv, ctx->num_sms, ctx->tune_sync, ctx->tune_wpg, bad, st));
+	if (prof_end(ctx, st)) return JPEGQS_ERR_CUDA;
+	ctx->launches++;
+	return 0;
+}
+
+/* de-quantize only (2551-2566) or clamp only (2670-2689) a whole component */
+static int launch_scale_clamp(jpegqs_cuda_ctx *ctx, const CompWork &w, int dequant, int clamp, cudaStream_t st) {
+	CK(qs_launch_scale_clamp(w.coef_dev, (size_t)w.W * w.H * 64, ctx->quant_dev + w.qslot, dequant, clamp, st));
+	ctx->launches++;
+	return 0;
+}
+
+/* per-component prelude of 2484-2566: the passes component w takes (niter2 smoothing iterations
+ * + the extra render pass); once `stop` is set it is de-quantized only.  Returns 1 when w
+ * iterates, 0 when not, or an error. */
+static int comp_prelude(jpegqs_cuda_ctx *ctx, ImgState &s, CompWork &w, int niter, cudaStream_t st) {
+	if (!w.c->has_qtbl) return 0;                                      /* 2494 */
+	w.extra = (s.image1 || (!w.ci && s.need_downsample)) ? 1 : 0;      /* 2495 */
+	w.niter2 = w.qval <= 1 ? 0 : niter;                                /* 2501 */
+	if (w.qval >= 0x800 && !s.stop) { s.stop = 1; s.stop_ci = w.ci; }  /* 2504 */
+	if (w.niter2 + w.extra == 0) return 0;                             /* 2542 */
+	if (s.stop) return launch_scale_clamp(ctx, w, 1, 0, st);           /* 2551-2566 */
+	if (!(w.W * w.H)) return 0;
+	w.iterate = true;
+	return 1;
+}
+
+/* post step of chroma component w: upsample_row + FDCT (2691-2752) into its luma-sized
+ * coefficients.  y_row0_px: first luma pixel row of the slab inside the image */
+static int post_upsample(jpegqs_cuda_ctx *ctx, const ImgState &s, const CompWork &w, int y_row0_px, cudaStream_t st) {
+	const jpegqs_cuda_image *im = s.im;
+	int ws = im->comp[0].h_samp, hs = im->comp[0].v_samp;
+	int w1 = ((int)im->image_width + ws - 1) / ws, h1 = ((int)im->image_height + hs - 1) / hs;
+	int W0 = im->comp[0].wblk, H0 = im->comp[0].hblk;
+	uint8_t *mem = s.mem_buf[w.ci - 1];
+	CK(qs_launch_upsample(w.plane, s.image2, QS_PLANE_STRIDE(w.W), s.image1, QS_PLANE_STRIDE(W0),
+			mem, W0 * 8, w1, h1, ws, hs, W0 * 8, H0 * 8, y_row0_px, st));
+	CK(qs_launch_fdct_plane(mem, W0 * 8, s.coef_up_dev[w.ci - 1], W0, H0, st));
+	ctx->launches += 2;
+	return 0;
+}
+
+/* post step of the luma component w: the down-sampled luma plane of 2753-2815 into s.image2_buf,
+ * for the chroma block rows this slab holds.  Rows are addressed inside the whole components:
+ * y_row0 / c_row0 = first luma / chroma block row of the slab, *_hblk_total = block rows of the
+ * whole component.  At an image edge (top / bottom) the replicated border row is written too;
+ * interior halo rows come from the neighbours. */
+static int post_downsample(jpegqs_cuda_ctx *ctx, const ImgState &s, const CompWork &w, int y_row0, int y_hblk_total,
+		int c_row0, int c_hblk_total, bool top, bool bottom, cudaStream_t st) {
+	const jpegqs_cuda_comp *cc = &s.im->comp[1];
+	int ws = w.c->h_samp, hs = w.c->v_samp;
+	int h = y_hblk_total * 8, h2 = c_hblk_total * 8, h1_total = (h + hs - 1) / hs;
+	int first = top ? -1 : c_row0 * 8;
+	int last = bottom ? h2 : (c_row0 + (int)cc->hblk) * 8 - 1;
+	int dstride = QS_PLANE_STRIDE(cc->wblk);
+	if (last < first) return 0;
+	CK(qs_launch_downsample(w.plane, QS_PLANE_STRIDE(w.W), w.W * 8, h,
+			s.image2_buf + (size_t)(first - c_row0 * 8 + 1) * dstride, dstride, (int)cc->wblk * 8, h2,
+			ws, hs, y_row0 * 8, first, last - first + 1, h1_total, st));
+	ctx->launches++;
+	return 0;
+}
+
+/* end of an image (2834-2859): quant tables := 1, chroma replaced by the up-sampled arrays */
+static void image_finish(jpegqs_cuda_image *im, bool upsampled) {
+	for (int ci = 0; ci < im->ncomp; ci++)
+		if (im->comp[ci].has_qtbl) for (int k = 0; k < 64; k++) im->comp[ci].quant[k] = 1;
+	im->upsampled = upsampled ? 1 : 0;
+}
+
+/* end of a run (ev1 recorded): everything has landed in the caller's memory; device time and
+ * per-kernel timing */
+static int run_end(jpegqs_cuda_ctx *ctx, HostIo &io, bool on_device, cudaStream_t st) {
+	CK(cudaStreamSynchronize(st));
+	if (!on_device && io.finish()) return JPEGQS_ERR_CUDA;       /* the last scatter has finished */
+	CK(cudaEventElapsedTime(&ctx->last_ms, ctx->ev0, ctx->ev1));
+	if (prof_collect(ctx)) return JPEGQS_ERR_CUDA;
+	return 0;
+}
+
+/* ------------------------------------------------------------------------------------------
+ * whole-image driver
+ * ------------------------------------------------------------------------------------------ */
 /* Host entry points, one large image: a group's block rows are cut into slabs of about one
  * wave of the persistent smoothing kernel.  Iteration 0 then follows the upload slab by slab
  * (IDCT pass of slab k, smoothing of slab k-1 - which needs the first pixel row of slab k), and
  * the last iteration hands its slabs to the download as they finish, so that only the first
  * slab's upload and the last slab's download are not hidden behind kernels.  Results do not
  * depend on this: a pass reads only start-of-pass neighbour pixels (quantsmooth.h:1396-1401). */
-#define QS_MAX_SLABS 16
 struct SlabPlan { int K; int r[QS_MAX_SLABS + 1]; };
 
 static int run_images(jpegqs_cuda_ctx *ctx, int nimg, jpegqs_cuda_image *imgs, int flags, int niter,
@@ -731,120 +1013,25 @@ static int run_images(jpegqs_cuda_ctx *ctx, int nimg, jpegqs_cuda_image *imgs, i
 		cudaStream_t st) {
 	if (!ctx || nimg < 0 || (nimg && !imgs)) return JPEGQS_ERR_ARG;
 	if (progress && nimg != 1) return JPEGQS_ERR_ARG;
-	CK(cudaSetDevice(ctx->device));
-	ctx->launches = 0; ctx->last_ms = 0;
-	ctx->ev_kind.clear(); ctx->ev_used = 0;
-	if (niter < 0) niter = 0;
-	if (niter > 100) niter = 100;                       /* quantsmooth.h:2455-2456 */
+	if (run_start(ctx, &niter)) return JPEGQS_ERR_CUDA;
 
 	std::vector<ImgState> S(nimg);
-	std::vector<CompWork> all;
-	size_t bytes = 0, stage_bytes = 0; int nquant = 0, max_groups = 0;
-	if (ctx->up) ctx->up->drain();                      /* nothing of an earlier (failed) call may linger */
-	if (ctx->down) ctx->down->drain();
-	ctx->io_ev_used = 0;
+	std::vector<std::vector<CompWork> > W(nimg);
+	int max_groups = 0;
 	for (int n = 0; n < nimg; n++) {
-		jpegqs_cuda_image *im = &imgs[n]; ImgState &s = S[n];
-		memset(&s, 0, sizeof(s)); s.im = im; im->upsampled = 0; s.stop_ci = 1 << 30;
-		if (im->ncomp < 1 || im->ncomp > JPEGQS_CUDA_MAX_COMP) return JPEGQS_ERR_ARG;
-		s.need_downsample = (flags & (QS_JOINT_YUV | QS_UPSAMPLE_UV)) && im->is_ycbcr && im->ncomp >= 3 &&
-				im->comp[1].h_samp == 1 && im->comp[1].v_samp == 1 &&
-				im->comp[2].h_samp == 1 && im->comp[2].v_samp == 1;          /* 2447-2453 */
-		s.skip = niter <= 0 && !((flags & QS_UPSAMPLE_UV) && s.need_downsample);   /* 2458 */
+		ImgState &s = S[n];
 		if (ret) ret[n] = 0;
+		int rc = image_start(s, &imgs[n], flags, niter);
+		if (rc) return rc;
 		if (s.skip) continue;
-		if (s.need_downsample && (im->comp[1].wblk != im->comp[2].wblk || im->comp[1].hblk != im->comp[2].hblk))
-			return JPEGQS_ERR_ARG;
-		for (int ci = 0; ci < im->ncomp; ci++) {
-			jpegqs_cuda_comp *c = &im->comp[ci];
-			bool have = c->coef || (!on_device && c->rows);
-			if (!have && c->wblk && c->hblk) return JPEGQS_ERR_ARG;
-			size_t cb = (size_t)c->wblk * c->hblk * 128;
-			if (!on_device) {
-				bytes += align256(cb);
-				if (c->rows || !is_pinned(c->coef)) stage_bytes += align256(cb);
-			}
-			bytes += align256(QS_PLANE_BYTES(c->wblk, c->hblk));
-			nquant++;
-		}
-		bool sub = s.need_downsample && !(im->comp[0].h_samp == 1 && im->comp[0].v_samp == 1);
-		if (sub) {
-			bytes += align256(QS_PLANE_BYTES(im->comp[1].wblk, im->comp[1].hblk));
-			if (flags & QS_UPSAMPLE_UV) for (int j = 0; j < 2; j++) {
-				jpegqs_cuda_comp *c = &im->comp[1 + j];
-				if (!c->coef_up && !(!on_device && c->rows_up)) return JPEGQS_ERR_ARG;
-				size_t yb = (size_t)im->comp[0].wblk * im->comp[0].hblk;
-				bytes += align256(yb * 64);                 /* up-sampled pixel plane */
-				if (!on_device) {
-					bytes += align256(yb * 128);
-					if (c->rows_up || !is_pinned(c->coef_up)) stage_bytes += align256(yb * 128);
-				}
-			}
-		}
 		/* host buffers: luma and chroma are separate phases even when independent, so that the
 		 * chroma upload and the luma download overlap with compute (copy stream + events) */
-		s.ngroups = progress ? im->ncomp : ((s.need_downsample || (!on_device && im->ncomp > 1)) ? 2 : 1);
+		s.ngroups = progress ? s.im->ncomp : ((s.need_downsample || (!on_device && s.im->ncomp > 1)) ? 2 : 1);
 		if (s.ngroups > max_groups) max_groups = s.ngroups;
 	}
-	if (arena_reserve(ctx, bytes + 4096)) return JPEGQS_ERR_CUDA;
-	if (quant_reserve(ctx, nquant)) return JPEGQS_ERR_CUDA;
-	if (stage_bytes && stage_reserve(ctx, stage_bytes)) return JPEGQS_ERR_CUDA;
-	size_t stage_pos = 0;
-	auto stage_take = [&](size_t b) { char *p = ctx->stage + stage_pos; stage_pos += align256(b); return (int16_t *)p; };
-	/* block-row tables made up for flat pageable arrays (one pointer per block row) */
-	std::vector<std::unique_ptr<int16_t *[]> > rowstore;
-	auto flat_rows = [&](int16_t *base, uint32_t wblk, uint32_t hblk) -> int16_t *const * {
-		rowstore.emplace_back(new int16_t *[hblk ? hblk : 1]);
-		int16_t **t = rowstore.back().get();
-		for (uint32_t y = 0; y < hblk; y++) t[y] = base + (size_t)y * wblk * 64;
-		return t;
-	};
-
-	/* carve device memory, upload coefficients and quant constants */
-	std::vector<QsQuantDev> qhost; qhost.reserve(nquant);
-	std::vector<std::vector<CompWork> > W(nimg);
-	std::vector<std::vector<int> > qval(nimg);
-	for (int n = 0; n < nimg; n++) {
-		ImgState &s = S[n]; jpegqs_cuda_image *im = s.im;
-		if (s.skip) continue;
-		W[n].resize(im->ncomp); qval[n].resize(im->ncomp);
-		for (int ci = 0; ci < im->ncomp; ci++) {
-			jpegqs_cuda_comp *c = &im->comp[ci]; CompWork &w = W[n][ci];
-			memset(&w, 0, sizeof(w));
-			w.img = n; w.ci = ci; w.c = c; w.W = c->wblk; w.H = c->hblk;
-			w.luma = !ci || !im->is_ycbcr;                                /* 2639 */
-			size_t cb = (size_t)c->wblk * c->hblk * 128;
-			if (on_device) w.coef_dev = c->coef;
-			else {
-				w.coef_dev = (int16_t *)arena_take(ctx, cb);
-				if (c->rows) { w.rows = c->rows; w.pin = stage_take(cb); }
-				else if (is_pinned(c->coef)) { w.rows = NULL; w.pin = c->coef; }
-				else { w.rows = flat_rows(c->coef, c->wblk, c->hblk); w.pin = stage_take(cb); }
-			}
-			w.plane = (uint8_t *)arena_take(ctx, QS_PLANE_BYTES(c->wblk, c->hblk));
-			w.qslot = (int)qhost.size();
-			QsQuantDev q; quant_prepare(c->quant, &q, &qval[n][ci], ctx->tune_maxn, ctx->tune_uni, ctx->tune_merge); qhost.push_back(q);
-		}
-		bool sub = s.need_downsample && !(im->comp[0].h_samp == 1 && im->comp[0].v_samp == 1);
-		if (sub) {
-			s.image2_buf = (uint8_t *)arena_take(ctx, QS_PLANE_BYTES(im->comp[1].wblk, im->comp[1].hblk));
-			if (flags & QS_UPSAMPLE_UV) for (int j = 0; j < 2; j++) {
-				size_t yb = (size_t)im->comp[0].wblk * im->comp[0].hblk;
-				s.mem_buf[j] = (uint8_t *)arena_take(ctx, yb * 64);
-				s.coef_up_dev[j] = on_device ? im->comp[1 + j].coef_up : (int16_t *)arena_take(ctx, yb * 128);
-				if (!on_device) {
-					jpegqs_cuda_comp *c = &im->comp[1 + j]; CompWork &w = W[n][1 + j];
-					if (c->rows_up) { w.rows_up = c->rows_up; w.pin_up = stage_take(yb * 128); }
-					else if (is_pinned(c->coef_up)) { w.rows_up = NULL; w.pin_up = c->coef_up; }
-					else { w.rows_up = flat_rows(c->coef_up, im->comp[0].wblk, im->comp[0].hblk); w.pin_up = stage_take(yb * 128); }
-				}
-			}
-		}
-	}
-	assign_sched_slots(qhost.data(), (int)qhost.size());
-	if (!qhost.empty())
-		CK(cudaMemcpyAsync(ctx->quant_dev, qhost.data(), qhost.size() * sizeof(QsQuantDev), cudaMemcpyHostToDevice, st));
-	ctx->jobs_cache[0].clear(); ctx->jobs_cache[1].clear();
+	/* carve device memory, upload quant constants */
+	Layout ly(ctx, on_device);
+	{ int rc = run_layout(ly, S.data(), W.data(), nimg, flags, st); if (rc) return rc; }
 
 	auto group_range = [&](const ImgState &s, int g, int *c0, int *c1) {
 		if (progress) { *c0 = g; *c1 = g + 1; }
@@ -858,17 +1045,8 @@ static int run_images(jpegqs_cuda_ctx *ctx, int nimg, jpegqs_cuda_image *imgs, i
 	HostIo io(ctx);
 	std::vector<int> unit_of_group(max_groups > 0 ? max_groups : 1, -1);
 	std::vector<std::vector<int> > unit_of_slab(max_groups > 0 ? max_groups : 1);
-	auto seg_of = [&](const CompWork &w, int r0, int r1) {
-		IoSeg sg; sg.dev = w.coef_dev; sg.pin = w.pin; sg.rows = w.rows; sg.wblk = w.W; sg.r0 = r0; sg.r1 = r1;
-		return sg;
-	};
 	if (!on_device) {
-		while ((int)ctx->sync_ev.size() < 2 * max_groups) {
-			cudaEvent_t e; CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming)); ctx->sync_ev.push_back(e);
-		}
-		while ((int)ctx->slab_ev.size() < 2 * max_groups * QS_MAX_SLABS) {
-			cudaEvent_t e; CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming)); ctx->slab_ev.push_back(e);
-		}
+		if (group_events(ctx, max_groups)) return JPEGQS_ERR_CUDA;
 		for (int g = 0; g < max_groups; g++) {
 			if (nimg == 1 && !progress && ctx->tune_slabs && !ctx->tune_x2 && !(flags & QS_LOW_QUALITY) &&
 					!S[0].skip && g < S[0].ngroups && niter >= 1) {
@@ -878,7 +1056,7 @@ static int run_images(jpegqs_cuda_ctx *ctx, int nimg, jpegqs_cuda_image *imgs, i
 				bool ok = c1 > c0;
 				for (int ci = c0; ci < c1 && ok; ci++) {
 					CompWork &w = W[0][ci];
-					ok = w.c->has_qtbl && qval[0][ci] > 1 && qval[0][ci] < 0x800 && w.W > 0 && w.H > 0 &&
+					ok = w.c->has_qtbl && w.qval > 1 && w.qval < 0x800 && w.W > 0 && w.H > 0 &&
 							w.W == W[0][c0].W && w.H == W[0][c0].H;
 				}
 				if (ok) {
@@ -901,7 +1079,7 @@ static int run_images(jpegqs_cuda_ctx *ctx, int nimg, jpegqs_cuda_image *imgs, i
 				int c0, c1; group_range(S[0], g, &c0, &c1);
 				for (int k = 0; k < plan[g].K; k++) {
 					std::vector<IoSeg> segs;
-					for (int ci = c0; ci < c1; ci++) segs.push_back(seg_of(W[0][ci], plan[g].r[k], plan[g].r[k + 1]));
+					for (int ci = c0; ci < c1; ci++) segs.push_back(coef_seg(W[0][ci], plan[g].r[k], plan[g].r[k + 1]));
 					unit_of_slab[g].push_back(io.add_unit(std::move(segs), ctx->slab_ev[(2 * g) * QS_MAX_SLABS + k]));
 				}
 				unit_of_group[g] = unit_of_slab[g].back();
@@ -912,17 +1090,14 @@ static int run_images(jpegqs_cuda_ctx *ctx, int nimg, jpegqs_cuda_image *imgs, i
 				ImgState &s = S[n];
 				if (s.skip || g >= s.ngroups) continue;
 				int c0, c1; group_range(s, g, &c0, &c1);
-				for (int ci = c0; ci < c1; ci++) if (W[n][ci].W && W[n][ci].H) segs.push_back(seg_of(W[n][ci], 0, W[n][ci].H));
+				for (int ci = c0; ci < c1; ci++) if (W[n][ci].W && W[n][ci].H) segs.push_back(coef_seg(W[n][ci], 0, W[n][ci].H));
 			}
 			unit_of_group[g] = io.add_unit(std::move(segs), ctx->sync_ev[2 * g]);
 		}
 		if (io.start()) return JPEGQS_ERR_CUDA;
 	}
-	auto up_wait = [&](int unit) -> int { return io.wait(unit, st); };
-	auto download = [&](std::vector<IoSeg> segs, cudaEvent_t after) -> int { return io.download(std::move(segs), after); };
 
-	const float *tabs = (flags & QS_DIAGONALS) ? ctx->tab_diag : ctx->tab_plain;
-	int *bad_dev = ctx->flags_dev, *tile_counter = ctx->flags_dev + QS_MAX_JOBS;
+	int *bad_dev = ctx->flags_dev;
 	CK(cudaEventRecord(ctx->ev0, st));
 
 	/* progress bookkeeping, quantsmooth.h:2474-2482 (single image only) */
@@ -935,40 +1110,18 @@ static int run_images(jpegqs_cuda_ctx *ctx, int nimg, jpegqs_cuda_image *imgs, i
 		prog_thr = progprec ? (int)((unsigned)(prog_max + progprec - 1) / (unsigned)progprec) : 0;
 	}
 
-	auto make_job = [&](const CompWork &w, const uint8_t *plane2) {
-		QsJob j; memset(&j, 0, sizeof(j));
-		j.coef = w.coef_dev; j.plane = w.plane; j.plane2 = plane2;
-		j.quant = ctx->quant_dev + w.qslot;
-		j.wblk = w.W; j.hblk = w.H; j.stride = QS_PLANE_STRIDE(w.W); j.nblocks = w.W * w.H;
-		j.luma = w.luma; j.top_edge = 1; j.bottom_edge = 1;
-		return j;
-	};
-	auto make_slab_job = [&](const CompWork &w, const uint8_t *plane2, int r0, int r1) {
-		QsJob j = make_job(w, plane2);
+	auto slab_job = [&](const CompWork &w, const uint8_t *plane2, int r0, int r1) {
+		QsJob j = make_job(ctx, w, plane2, r0 == 0, r1 == w.H);
 		size_t poff = (size_t)r0 * 8 * j.stride;
 		j.coef += (size_t)r0 * w.W * 64; j.plane += poff;
 		if (plane2) j.plane2 += poff;
 		j.hblk = r1 - r0; j.nblocks = w.W * (r1 - r0);
-		j.top_edge = r0 == 0; j.bottom_edge = r1 == w.H;
 		return j;
-	};
-	auto launch_smooth = [&](const QsJob *jd, int nj, int tiles, int clampv) -> int {
-		if (prof_begin(ctx, 1, st)) return JPEGQS_ERR_CUDA;
-		if (flags & QS_LOW_QUALITY) CK(qs_launch_lowq(jd, nj, tiles, flags, clampv, NULL, st));
-#ifdef QS_EXPERIMENTS
-		else if (ctx->tune_x2) CK(qs_launch_smooth_x2(jd, nj, tiles,
-				(flags & QS_DIAGONALS) ? ctx->tab2_diag : ctx->tab2_plain, ctx->nslots2, tile_counter, flags, clampv,
-				ctx->num_sms, ctx->tune_sync, st));
-#endif
-		else CK(qs_launch_smooth(jd, nj, tiles, tabs, tile_counter, flags, clampv, ctx->num_sms, ctx->tune_sync, ctx->tune_wpg, NULL, st));
-		if (prof_end(ctx, st)) return JPEGQS_ERR_CUDA;
-		ctx->launches++;
-		return 0;
 	};
 
 	for (int g = 0; g < max_groups; g++) {
 		bool slab_in = !on_device && plan[g].K > 0 && !S[0].stop;
-		if (!on_device && !slab_in && up_wait(unit_of_group[g])) return JPEGQS_ERR_CUDA;
+		if (!on_device && !slab_in && io.wait(unit_of_group[g], st)) return JPEGQS_ERR_CUDA;
 		/* ---- which components belong to this phase; per-component prelude 2484-2566 ---- */
 		std::vector<CompWork *> works;
 		int prog_cur = 0, prog_inc = 0;
@@ -979,38 +1132,24 @@ static int run_images(jpegqs_cuda_ctx *ctx, int nimg, jpegqs_cuda_image *imgs, i
 			for (int ci = c0; ci < c1; ci++) {
 				CompWork &w = W[n][ci];
 				if (progress) { prog_cur = prog_next; prog_inc = w.c->v_samp; prog_next += w.H * prog_inc * niter; }
-				if (!w.c->has_qtbl) continue;                              /* 2494 */
-				w.extra = (s.image1 || (!ci && s.need_downsample)) ? 1 : 0;      /* 2495 */
-				w.niter2 = qval[n][ci] <= 1 ? 0 : niter;                   /* 2501 */
-				if (qval[n][ci] >= 0x800 && !s.stop) { s.stop = 1; s.stop_ci = ci; }   /* 2504 */
-				if (w.niter2 + w.extra == 0) continue;                     /* 2542 */
-				if (s.stop) {                                              /* 2551-2566 */
-					CK(qs_launch_scale_clamp(w.coef_dev, (size_t)w.W * w.H * 64, ctx->quant_dev + w.qslot, 1, 0, st));
-					ctx->launches++;
-					continue;
-				}
-				if (!(w.W * w.H)) continue;
-				w.iterate = true;
-				works.push_back(&w);
+				int rc = comp_prelude(ctx, s, w, niter, st);
+				if (rc < 0) return rc;
+				if (rc) works.push_back(&w);
 			}
 		}
 
 		int max_pass = 0;
 		for (CompWork *w : works) if (w->niter2 + w->extra > max_pass) max_pass = w->niter2 + w->extra;
-		auto p2_of = [&](const CompWork *w) -> const uint8_t * {
-			ImgState &s = S[w->img];
-			return (s.image2 && (flags & QS_JOINT_YUV) && w->ci > 0) ? s.image2 : NULL;
-		};
 		if (slab_in) {
 			int c0, c1; group_range(S[0], g, &c0, &c1);
 			bool ok = (int)works.size() == c1 - c0;
 			for (CompWork *w : works) ok = ok && w->niter2 == works[0]->niter2 && w->extra == works[0]->extra && w->niter2 >= 1;
-			if (!ok) { slab_in = false; if (up_wait(unit_of_group[g])) return JPEGQS_ERR_CUDA; }
+			if (!ok) { slab_in = false; if (io.wait(unit_of_group[g], st)) return JPEGQS_ERR_CUDA; }
 		}
 		/* the download pipeline needs the slab plan but not the upload pipeline, and vice versa:
 		 * a middle group's transfers hide behind its neighbours' kernels anyway */
 		bool slab_out = slab_in && works[0]->niter2 >= 2 && !works[0]->extra && g == S[0].ngroups - 1;
-		if (slab_in && g > 0) { slab_in = false; if (up_wait(unit_of_group[g])) return JPEGQS_ERR_CUDA; }
+		if (slab_in && g > 0) { slab_in = false; if (io.wait(unit_of_group[g], st)) return JPEGQS_ERR_CUDA; }
 		for (int iter = 0; iter < max_pass; iter++) {
 			if (iter == 0 && slab_in) {
 				/* ---- iteration 0 behind the upload, slab by slab ---- */
@@ -1018,22 +1157,16 @@ static int run_images(jpegqs_cuda_ctx *ctx, int nimg, jpegqs_cuda_image *imgs, i
 				int cl = (works[0]->niter2 == 1 && !works[0]->extra) ? 1 : 0;
 				CK(cudaMemsetAsync(bad_dev, 0, works.size() * sizeof(int), st));
 				for (int k = 0; k <= pl.K; k++) {
-					const QsJob *jd; int tiles;
 					if (k < pl.K) {
-						if (up_wait(unit_of_slab[g][k])) return JPEGQS_ERR_CUDA;
+						if (io.wait(unit_of_slab[g][k], st)) return JPEGQS_ERR_CUDA;
 						std::vector<QsJob> jobs;
-						for (CompWork *w : works) jobs.push_back(make_slab_job(*w, NULL, pl.r[k], pl.r[k + 1]));
-						if (upload_jobs(ctx, 0, jobs, st, &jd, &tiles)) return JPEGQS_ERR_CUDA;
-						if (prof_begin(ctx, 0, st)) return JPEGQS_ERR_CUDA;
-						CK(qs_launch_idct_pass(jd, (int)jobs.size(), tiles, QS_IDCT_DEQUANT, bad_dev, st));
-						if (prof_end(ctx, st)) return JPEGQS_ERR_CUDA;
-						ctx->launches++;
+						for (CompWork *w : works) jobs.push_back(slab_job(*w, NULL, pl.r[k], pl.r[k + 1]));
+						if (launch_idct(ctx, jobs, QS_IDCT_DEQUANT, false, st)) return JPEGQS_ERR_CUDA;
 					}
 					if (k >= 1) {
 						std::vector<QsJob> jobs;
-						for (CompWork *w : works) jobs.push_back(make_slab_job(*w, p2_of(w), pl.r[k - 1], pl.r[k]));
-						if (upload_jobs(ctx, 1, jobs, st, &jd, &tiles)) return JPEGQS_ERR_CUDA;
-						if (launch_smooth(jd, (int)jobs.size(), tiles, cl)) return JPEGQS_ERR_CUDA;
+						for (CompWork *w : works) jobs.push_back(slab_job(*w, plane2_of(S[0], *w, flags), pl.r[k - 1], pl.r[k]));
+						if (launch_smooth(ctx, jobs, flags, cl, false, st)) return JPEGQS_ERR_CUDA;
 					}
 				}
 				CK(qs_copy_flags(bad_dev, ctx->flags_host, (int)works.size(), st));
@@ -1061,17 +1194,12 @@ static int run_images(jpegqs_cuda_ctx *ctx, int nimg, jpegqs_cuda_image *imgs, i
 					if (!w->iterate || iter >= w->niter2 + w->extra) continue;
 					int cl = (iter == w->niter2) ? 1 : 0;
 					if (cl != clampv) continue;
-					jobs.push_back(make_job(*w, NULL)); who.push_back(w);
+					jobs.push_back(make_job(ctx, *w, NULL, 1, 1)); who.push_back(w);
 				}
 				if (jobs.empty()) continue;
-				const QsJob *jd; int tiles;
-				if (upload_jobs(ctx, 0, jobs, st, &jd, &tiles)) return JPEGQS_ERR_CUDA;
 				int mode = (iter == 0 ? QS_IDCT_DEQUANT : 0) | (clampv ? QS_IDCT_CLAMP : 0);
 				if (iter == 0) CK(cudaMemsetAsync(bad_dev, 0, jobs.size() * sizeof(int), st));
-				if (prof_begin(ctx, 0, st)) return JPEGQS_ERR_CUDA;
-				CK(qs_launch_idct_pass(jd, (int)jobs.size(), tiles, mode, bad_dev, st));
-				if (prof_end(ctx, st)) return JPEGQS_ERR_CUDA;
-				ctx->launches++;
+				if (launch_idct(ctx, jobs, mode, false, st)) return JPEGQS_ERR_CUDA;
 				if (clampv) for (CompWork *w : who) w->done_clamp = true;
 				if (iter == 0) {                                           /* bad_coef, 2602-2610 */
 					CK(qs_copy_flags(bad_dev, ctx->flags_host, (int)jobs.size(), st));
@@ -1097,15 +1225,13 @@ static int run_images(jpegqs_cuda_ctx *ctx, int nimg, jpegqs_cuda_image *imgs, i
 				const SlabPlan &pl = plan[g];
 				for (int k = 0; k < pl.K; k++) {
 					std::vector<QsJob> jobs;
-					for (CompWork *w : works) jobs.push_back(make_slab_job(*w, p2_of(w), pl.r[k], pl.r[k + 1]));
-					const QsJob *jd; int tiles;
-					if (upload_jobs(ctx, 1, jobs, st, &jd, &tiles)) return JPEGQS_ERR_CUDA;
-					if (launch_smooth(jd, (int)jobs.size(), tiles, 1)) return JPEGQS_ERR_CUDA;
+					for (CompWork *w : works) jobs.push_back(slab_job(*w, plane2_of(S[0], *w, flags), pl.r[k], pl.r[k + 1]));
+					if (launch_smooth(ctx, jobs, flags, 1, false, st)) return JPEGQS_ERR_CUDA;
 					cudaEvent_t e = ctx->slab_ev[(2 * g + 1) * QS_MAX_SLABS + k];
 					CK(cudaEventRecord(e, st));
 					std::vector<IoSeg> segs;
-					for (CompWork *w : works) segs.push_back(seg_of(*w, pl.r[k], pl.r[k + 1]));
-					if (download(std::move(segs), e)) return JPEGQS_ERR_CUDA;
+					for (CompWork *w : works) segs.push_back(coef_seg(*w, pl.r[k], pl.r[k + 1]));
+					if (io.download(std::move(segs), e)) return JPEGQS_ERR_CUDA;
 				}
 				for (CompWork *w : works) { w->done_clamp = true; w->downloaded = true; }
 				continue;
@@ -1116,12 +1242,10 @@ static int run_images(jpegqs_cuda_ctx *ctx, int nimg, jpegqs_cuda_image *imgs, i
 					if (!w->iterate || iter >= w->niter2) continue;
 					int cl = (iter == w->niter2 - 1 && !w->extra) ? 1 : 0;
 					if (cl != clampv) continue;
-					jobs.push_back(make_job(*w, p2_of(w))); who.push_back(w);
+					jobs.push_back(make_job(ctx, *w, plane2_of(S[w->img], *w, flags), 1, 1)); who.push_back(w);
 				}
 				if (jobs.empty()) continue;
-				const QsJob *jd; int tiles;
-				if (upload_jobs(ctx, 1, jobs, st, &jd, &tiles)) return JPEGQS_ERR_CUDA;
-				if (launch_smooth(jd, (int)jobs.size(), tiles, clampv)) return JPEGQS_ERR_CUDA;
+				if (launch_smooth(ctx, jobs, flags, clampv, false, st)) return JPEGQS_ERR_CUDA;
 				if (clampv) for (CompWork *w : who) w->done_clamp = true;
 			}
 			if (progress && works.size() == 1 && works[0]->iterate && iter < works[0]->niter2) {   /* 2656-2664 */
@@ -1139,32 +1263,20 @@ static int run_images(jpegqs_cuda_ctx *ctx, int nimg, jpegqs_cuda_image *imgs, i
 		}
 		/* ---- components that left the loop early still get the clamp of 2670-2689 ---- */
 		for (CompWork *w : works) if (!w->done_clamp) {
-			CK(qs_launch_scale_clamp(w->coef_dev, (size_t)w->W * w->H * 64, ctx->quant_dev + w->qslot, 0, 1, st));
-			ctx->launches++; w->done_clamp = true;
+			if (launch_scale_clamp(ctx, *w, 0, 1, st)) return JPEGQS_ERR_CUDA;
+			w->done_clamp = true;
 		}
 		/* ---- post steps: chroma up-sampling (2691-2752), luma planes (2753-2815) ---- */
 		for (CompWork *w : works) {
-			ImgState &s = S[w->img]; jpegqs_cuda_image *im = s.im;
+			ImgState &s = S[w->img];
 			if (s.stop) continue;
 			if (w->ci > 0 && s.image1 && w->ci <= 2) {
-				int ws = im->comp[0].h_samp, hs = im->comp[0].v_samp;
-				int w1 = (im->image_width + ws - 1) / ws, h1 = (im->image_height + hs - 1) / hs;
-				int W0 = im->comp[0].wblk, H0 = im->comp[0].hblk;
-				uint8_t *mem = s.mem_buf[w->ci - 1];
-				CK(qs_launch_upsample(w->plane, s.image2, QS_PLANE_STRIDE(w->W), s.image1, QS_PLANE_STRIDE(W0),
-						mem, W0 * 8, w1, h1, ws, hs, W0 * 8, H0 * 8, 0, st));
-				CK(qs_launch_fdct_plane(mem, W0 * 8, s.coef_up_dev[w->ci - 1], W0, H0, st));
-				ctx->launches += 2;
+				if (post_upsample(ctx, s, *w, 0, st)) return JPEGQS_ERR_CUDA;
 			} else if (w->ci == 0 && s.need_downsample) {
-				int ws = w->c->h_samp, hs = w->c->v_samp;
-				if (ws == 1 && hs == 1) s.image2 = w->plane;
+				if (w->c->h_samp == 1 && w->c->v_samp == 1) s.image2 = w->plane;
 				else {
 					if (flags & QS_UPSAMPLE_UV) s.image1 = w->plane;
-					int w2 = im->comp[1].wblk * 8, h2 = im->comp[1].hblk * 8;
-					int h1 = (w->H * 8 + hs - 1) / hs;
-					CK(qs_launch_downsample(w->plane, QS_PLANE_STRIDE(w->W), w->W * 8, w->H * 8,
-							s.image2_buf, QS_PLANE_STRIDE(im->comp[1].wblk), w2, h2, ws, hs, 0, -1, h2 + 2, h1, st));
-					ctx->launches++;
+					if (post_downsample(ctx, s, *w, 0, w->H, 0, (int)s.im->comp[1].hblk, true, true, st)) return JPEGQS_ERR_CUDA;
 					s.image2 = s.image2_buf;
 				}
 			}
@@ -1174,41 +1286,26 @@ static int run_images(jpegqs_cuda_ctx *ctx, int nimg, jpegqs_cuda_image *imgs, i
 			CK(cudaEventRecord(ctx->sync_ev[2 * g + 1], st));
 			std::vector<IoSeg> segs;
 			for (int n = 0; n < nimg; n++) {
-				ImgState &s = S[n]; jpegqs_cuda_image *im = s.im;
+				ImgState &s = S[n];
 				if (s.skip || g >= s.ngroups) continue;
 				int c0, c1; group_range(s, g, &c0, &c1);
 				for (int ci = c0; ci < c1; ci++) {
 					CompWork &w = W[n][ci];
-					if (w.W && w.H && !w.downloaded) segs.push_back(seg_of(w, 0, w.H));
-					if (s.image1 && !s.stop && ci >= 1 && ci <= 2) {
-						IoSeg sg; sg.dev = s.coef_up_dev[ci - 1]; sg.pin = w.pin_up; sg.rows = w.rows_up;
-						sg.wblk = im->comp[0].wblk; sg.r0 = 0; sg.r1 = im->comp[0].hblk;
-						segs.push_back(sg);
-					}
+					if (w.W && w.H && !w.downloaded) segs.push_back(coef_seg(w, 0, w.H));
+					if (s.image1 && !s.stop && ci >= 1 && ci <= 2) segs.push_back(up_seg(s, w, 0, s.im->comp[0].hblk));
 				}
 			}
-			if (download(std::move(segs), ctx->sync_ev[2 * g + 1])) return JPEGQS_ERR_CUDA;
+			if (io.download(std::move(segs), ctx->sync_ev[2 * g + 1])) return JPEGQS_ERR_CUDA;
 		}
 	}
 	CK(cudaEventRecord(ctx->ev1, st));
-
-	/* ---- results ---- */
 	for (int n = 0; n < nimg; n++) {
-		ImgState &s = S[n]; jpegqs_cuda_image *im = s.im;
+		ImgState &s = S[n];
 		if (s.skip) continue;
-		bool ups = s.image1 && !s.stop;                                 /* 2834-2849 */
-		for (int ci = 0; ci < im->ncomp; ci++) {
-			CompWork &w = W[n][ci];
-			if (w.c->has_qtbl) for (int k = 0; k < 64; k++) w.c->quant[k] = 1;      /* 2851-2859 */
-		}
-		im->upsampled = ups ? 1 : 0;
+		image_finish(s.im, s.image1 && !s.stop);
 		if (ret) ret[n] = s.stop;
 	}
-	CK(cudaStreamSynchronize(st));
-	if (!on_device && io.finish()) return JPEGQS_ERR_CUDA;  /* the last scatter has finished */
-	CK(cudaEventElapsedTime(&ctx->last_ms, ctx->ev0, ctx->ev1));
-	if (prof_collect(ctx)) return JPEGQS_ERR_CUDA;
-	return 0;
+	return run_end(ctx, io, on_device, st);
 }
 
 extern "C" int jpegqs_cuda_run_host(jpegqs_cuda_ctx *ctx, jpegqs_cuda_image *img, int flags, int niter,
@@ -1423,8 +1520,7 @@ static int slab_exchange(jpegqs_cuda_ctx *ctx, jpegqs_cuda_link *l, const std::v
 }
 
 /* do_quantsmooth on ONE SLAB of an image: img describes the slab (comp[].hblk = block rows held
- * by this rank, coef / rows = those rows), geom where it sits.  The slab-local restatement of
- * run_images (itself the reference driver, quantsmooth.h:2404-2878); the schedule is
+ * by this rank, coef / rows = those rows), geom where it sits.  Unlike run_images the schedule is
  * unconditional - what the reference decides with `stop` is decided on the device from the
  * run's out-of-range flags (QsJob.stop_aware), which the ranks OR-combine in the first exchange
  * of a phase - so every rank issues the same exchanges whatever its data look like. */
@@ -1434,115 +1530,33 @@ static int run_slab(jpegqs_cuda_ctx *ctx, jpegqs_cuda_link *link, jpegqs_cuda_im
 	const int rank = link ? link->rank : 0, world = link ? link->world : 1;
 	if (link && (link->ctx != ctx || !link->connected)) return JPEGQS_ERR_ARG;
 	if (geom->rank != rank || geom->world != world) return JPEGQS_ERR_ARG;
-	CK(cudaSetDevice(ctx->device));
-	ctx->launches = 0; ctx->last_ms = 0; ctx->ev_kind.clear(); ctx->ev_used = 0;
-	if (niter < 0) niter = 0;
-	if (niter > 100) niter = 100;
-	const int nc = im->ncomp;
-	if (nc < 1 || nc > JPEGQS_CUDA_MAX_COMP) return JPEGQS_ERR_ARG;
+	if (run_start(ctx, &niter)) return JPEGQS_ERR_CUDA;
 	const bool top = rank == 0, bottom = rank == world - 1;
-	im->upsampled = 0;
 	if (ret) *ret = 0;
-	bool need_ds = (flags & (QS_JOINT_YUV | QS_UPSAMPLE_UV)) && im->is_ycbcr && nc >= 3 &&
-			im->comp[1].h_samp == 1 && im->comp[1].v_samp == 1 && im->comp[2].h_samp == 1 && im->comp[2].v_samp == 1;
-	if (niter <= 0 && !((flags & QS_UPSAMPLE_UV) && need_ds)) return 0;                   /* 2458 */
-	if (need_ds && (im->comp[1].wblk != im->comp[2].wblk || im->comp[1].hblk != im->comp[2].hblk)) return JPEGQS_ERR_ARG;
-	const bool sub = need_ds && !(im->comp[0].h_samp == 1 && im->comp[0].v_samp == 1);
-	const bool ups = sub && (flags & QS_UPSAMPLE_UV);
-	if (ctx->up) ctx->up->drain();
-	if (ctx->down) ctx->down->drain();
-	ctx->io_ev_used = 0;
-
-	/* ---- memory ---- */
-	size_t bytes = 0, stage_bytes = 0;
-	for (int ci = 0; ci < nc; ci++) {
-		jpegqs_cuda_comp *c = &im->comp[ci];
-		if (!(c->coef || (!on_device && c->rows)) && c->wblk && c->hblk) return JPEGQS_ERR_ARG;
-		if (world > 1 && (!c->hblk || !c->wblk)) {
-			snprintf(ctx->err, sizeof(ctx->err), "sharded run: rank %d holds no block row of component %d", rank, ci);
-			return JPEGQS_ERR_ARG;
-		}
-		size_t cb = (size_t)c->wblk * c->hblk * 128;
-		if (!on_device) { bytes += align256(cb); if (c->rows || !is_pinned(c->coef)) stage_bytes += align256(cb); }
-		bytes += align256(QS_PLANE_BYTES(c->wblk, c->hblk));
+	ImgState s;
+	{ int rc = image_start(s, im, flags, niter); if (rc) return rc; }
+	if (s.skip) return 0;
+	const int nc = im->ncomp;
+	for (int ci = 0; ci < nc && world > 1; ci++) if (!im->comp[ci].hblk || !im->comp[ci].wblk) {
+		snprintf(ctx->err, sizeof(ctx->err), "sharded run: rank %d holds no block row of component %d", rank, ci);
+		return JPEGQS_ERR_ARG;
 	}
-	const size_t yb = (size_t)im->comp[0].wblk * im->comp[0].hblk;
-	if (sub) {
-		bytes += align256(QS_PLANE_BYTES(im->comp[1].wblk, im->comp[1].hblk));
-		if (ups) for (int j = 0; j < 2; j++) {
-			jpegqs_cuda_comp *c = &im->comp[1 + j];
-			if (!c->coef_up && !(!on_device && c->rows_up)) return JPEGQS_ERR_ARG;
-			bytes += align256(yb * 64);
-			if (!on_device) { bytes += align256(yb * 128); if (c->rows_up || !is_pinned(c->coef_up)) stage_bytes += align256(yb * 128); }
-		}
-	}
-	if (arena_reserve(ctx, bytes + 4096)) return JPEGQS_ERR_CUDA;
-	if (quant_reserve(ctx, nc)) return JPEGQS_ERR_CUDA;
-	if (stage_bytes && stage_reserve(ctx, stage_bytes)) return JPEGQS_ERR_CUDA;
-	size_t stage_pos = 0;
-	auto stage_take = [&](size_t b) { char *p = ctx->stage + stage_pos; stage_pos += align256(b); return (int16_t *)p; };
-	std::vector<std::unique_ptr<int16_t *[]> > rowstore;
-	auto flat_rows = [&](int16_t *base, uint32_t wblk, uint32_t hblk) -> int16_t *const * {
-		rowstore.emplace_back(new int16_t *[hblk ? hblk : 1]);
-		int16_t **t = rowstore.back().get();
-		for (uint32_t y = 0; y < hblk; y++) t[y] = base + (size_t)y * wblk * 64;
-		return t;
-	};
-	std::vector<CompWork> W(nc); std::vector<QsQuantDev> qhost(nc); std::vector<int> qval(nc);
-	for (int ci = 0; ci < nc; ci++) {
-		jpegqs_cuda_comp *c = &im->comp[ci]; CompWork &w = W[ci];
-		memset(&w, 0, sizeof(w));
-		w.ci = ci; w.c = c; w.W = c->wblk; w.H = c->hblk; w.luma = !ci || !im->is_ycbcr; w.qslot = ci;
-		size_t cb = (size_t)c->wblk * c->hblk * 128;
-		if (on_device) w.coef_dev = c->coef;
-		else {
-			w.coef_dev = (int16_t *)arena_take(ctx, cb);
-			if (c->rows) { w.rows = c->rows; w.pin = stage_take(cb); }
-			else if (is_pinned(c->coef)) { w.rows = NULL; w.pin = c->coef; }
-			else { w.rows = flat_rows(c->coef, c->wblk, c->hblk); w.pin = stage_take(cb); }
-		}
-		w.plane = (uint8_t *)arena_take(ctx, QS_PLANE_BYTES(c->wblk, c->hblk));
-		quant_prepare(c->quant, &qhost[ci], &qval[ci], ctx->tune_maxn, ctx->tune_uni, ctx->tune_merge);
-	}
-	uint8_t *image2_buf = NULL, *mem_buf[2] = { NULL, NULL }; int16_t *coef_up_dev[2] = { NULL, NULL };
-	if (sub) {
-		image2_buf = (uint8_t *)arena_take(ctx, QS_PLANE_BYTES(im->comp[1].wblk, im->comp[1].hblk));
-		if (ups) for (int j = 0; j < 2; j++) {
-			jpegqs_cuda_comp *c = &im->comp[1 + j]; CompWork &w = W[1 + j];
-			mem_buf[j] = (uint8_t *)arena_take(ctx, yb * 64);
-			coef_up_dev[j] = on_device ? c->coef_up : (int16_t *)arena_take(ctx, yb * 128);
-			if (!on_device) {
-				if (c->rows_up) { w.rows_up = c->rows_up; w.pin_up = stage_take(yb * 128); }
-				else if (is_pinned(c->coef_up)) { w.rows_up = NULL; w.pin_up = c->coef_up; }
-				else { w.rows_up = flat_rows(c->coef_up, im->comp[0].wblk, im->comp[0].hblk); w.pin_up = stage_take(yb * 128); }
-			}
-		}
-	}
-	assign_sched_slots(qhost.data(), nc);
-	CK(cudaMemcpyAsync(ctx->quant_dev, qhost.data(), (size_t)nc * sizeof(QsQuantDev), cudaMemcpyHostToDevice, st));
-	ctx->jobs_cache[0].clear(); ctx->jobs_cache[1].clear();
+	Layout ly(ctx, on_device);
+	std::vector<CompWork> W;
+	{ int rc = run_layout(ly, &s, &W, 1, flags, st); if (rc) return rc; }
 
 	/* ---- phases (luma | chroma when the chroma needs the finished luma, or to overlap the
 	 *      transfers of host buffers), uploads ---- */
-	const int ngroups = (need_ds || (!on_device && nc > 1)) ? 2 : 1;
+	const int ngroups = (s.need_downsample || (!on_device && nc > 1)) ? 2 : 1;
 	auto group_range = [&](int g, int *c0, int *c1) {
 		if (ngroups == 2) { *c0 = g ? 1 : 0; *c1 = g ? nc : 1; } else { *c0 = 0; *c1 = nc; }
 	};
 	HostIo io(ctx);
 	int unit_of_group[2] = { -1, -1 }, nbands[2] = { 1, 1 };
-	auto seg_of = [&](const CompWork &w, int r0, int r1) {
-		IoSeg sg; sg.dev = w.coef_dev; sg.pin = w.pin; sg.rows = w.rows; sg.wblk = w.W; sg.r0 = r0; sg.r1 = r1;
-		return sg;
-	};
 	if (!on_device) {
-		while ((int)ctx->sync_ev.size() < 2 * ngroups) {
-			cudaEvent_t e; CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming)); ctx->sync_ev.push_back(e);
-		}
 		/* a phase travels in bands of ~8 MB: the H2D copy of band k runs while band k+1 is being
 		 * gathered (and, on the way back, band k is scattered while band k+1 is still in flight) */
-		while ((int)ctx->slab_ev.size() < 2 * ngroups * QS_MAX_SLABS) {
-			cudaEvent_t e; CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming)); ctx->slab_ev.push_back(e);
-		}
+		if (group_events(ctx, ngroups)) return JPEGQS_ERR_CUDA;
 		for (int g = 0; g < ngroups; g++) {
 			int c0, c1; group_range(g, &c0, &c1);
 			size_t gb = 0;
@@ -1552,7 +1566,7 @@ static int run_slab(jpegqs_cuda_ctx *ctx, jpegqs_cuda_link *link, jpegqs_cuda_im
 				std::vector<IoSeg> segs;
 				for (int ci = c0; ci < c1; ci++) {
 					int r0 = (int)((long)k * W[ci].H / nbands[g]), r1 = (int)((long)(k + 1) * W[ci].H / nbands[g]);
-					if (W[ci].W && r1 > r0) segs.push_back(seg_of(W[ci], r0, r1));
+					if (W[ci].W && r1 > r0) segs.push_back(coef_seg(W[ci], r0, r1));
 				}
 				unit_of_group[g] = io.add_unit(std::move(segs), k == nbands[g] - 1 ? ctx->sync_ev[2 * g] : ctx->slab_ev[(2 * g) * QS_MAX_SLABS + k]);
 			}
@@ -1560,47 +1574,26 @@ static int run_slab(jpegqs_cuda_ctx *ctx, jpegqs_cuda_link *link, jpegqs_cuda_im
 		if (io.start()) return JPEGQS_ERR_CUDA;
 	}
 
-	const float *tabs = (flags & QS_DIAGONALS) ? ctx->tab_diag : ctx->tab_plain;
-	int *bad_dev = ctx->flags_dev, *tile_counter = ctx->flags_dev + QS_MAX_JOBS;
+	int *bad_dev = ctx->flags_dev;
 	CK(cudaMemsetAsync(bad_dev, 0, 16 * sizeof(int), st));
 	CK(cudaEventRecord(ctx->ev0, st));
-	auto make_job = [&](const CompWork &w, const uint8_t *plane2) {
-		QsJob j; memset(&j, 0, sizeof(j));
-		j.coef = w.coef_dev; j.plane = w.plane; j.plane2 = plane2;
-		j.quant = ctx->quant_dev + w.qslot;
-		j.wblk = w.W; j.hblk = w.H; j.stride = QS_PLANE_STRIDE(w.W); j.nblocks = w.W * w.H;
-		j.luma = w.luma; j.top_edge = top; j.bottom_edge = bottom;
+	auto slab_job = [&](const CompWork &w, const uint8_t *plane2) {
+		QsJob j = make_job(ctx, w, plane2, top, bottom);
 		j.bad_slot = w.ci; j.bad_first = 0; j.stop_aware = 1;
 		return j;
 	};
-	int static_stop_ci = 1 << 30;                          /* quantsmooth.h:2504: a quant value >= 0x800 */
-	uint8_t *image1 = NULL, *image2 = NULL;
 
 	for (int g = 0; g < ngroups; g++) {
 		if (!on_device && io.wait(unit_of_group[g], st)) return JPEGQS_ERR_CUDA;
 		int c0, c1; group_range(g, &c0, &c1);
 		std::vector<CompWork *> works;
-		for (int ci = c0; ci < c1; ci++) {
-			CompWork &w = W[ci];
-			if (!w.c->has_qtbl) continue;                                  /* 2494 */
-			w.extra = (image1 || (!ci && need_ds)) ? 1 : 0;                /* 2495 */
-			w.niter2 = qval[ci] <= 1 ? 0 : niter;                          /* 2501 */
-			if (qval[ci] >= 0x800 && ci < static_stop_ci) static_stop_ci = ci;
-			if (w.niter2 + w.extra == 0) continue;                         /* 2542 */
-			if (ci >= static_stop_ci) {                                    /* 2551-2566 */
-				CK(qs_launch_scale_clamp(w.coef_dev, (size_t)w.W * w.H * 64, ctx->quant_dev + w.qslot, 1, 0, st));
-				ctx->launches++;
-				continue;
-			}
-			if (!(w.W * w.H)) continue;
-			w.iterate = true;
-			works.push_back(&w);
+		for (int ci = c0; ci < c1; ci++) {              /* only the static stop of 2504 is known on the host */
+			int rc = comp_prelude(ctx, s, W[ci], niter, st);
+			if (rc < 0) return rc;
+			if (rc) works.push_back(&W[ci]);
 		}
 		int max_pass = 0;
 		for (CompWork *w : works) max_pass = std::max(max_pass, w->niter2 + w->extra);
-		auto p2_of = [&](const CompWork *w) -> const uint8_t * {
-			return (image2 && (flags & QS_JOINT_YUV) && w->ci > 0) ? image2 : NULL;
-		};
 		for (int iter = 0; iter < max_pass; iter++) {
 			std::vector<XchgPlane> xp;
 			for (int clampv = 0; clampv < 2; clampv++) {                   /* IDCT pass, 2589-2620 (+ final clamp) */
@@ -1608,17 +1601,12 @@ static int run_slab(jpegqs_cuda_ctx *ctx, jpegqs_cuda_link *link, jpegqs_cuda_im
 				for (CompWork *w : works) {
 					if (iter >= w->niter2 + w->extra) continue;
 					if (((iter == w->niter2) ? 1 : 0) != clampv) continue;
-					jobs.push_back(make_job(*w, NULL));
+					jobs.push_back(slab_job(*w, NULL));
 					xp.push_back({ w->plane, w->W, w->H });
 				}
 				if (jobs.empty()) continue;
-				const QsJob *jd; int tiles;
-				if (upload_jobs(ctx, 0, jobs, st, &jd, &tiles, true)) return JPEGQS_ERR_CUDA;
 				int mode = (iter == 0 ? QS_IDCT_DEQUANT : 0) | (clampv ? QS_IDCT_CLAMP : 0);
-				if (prof_begin(ctx, 0, st)) return JPEGQS_ERR_CUDA;
-				CK(qs_launch_idct_pass(jd, (int)jobs.size(), tiles, mode, bad_dev, st));
-				if (prof_end(ctx, st)) return JPEGQS_ERR_CUDA;
-				ctx->launches++;
+				if (launch_idct(ctx, jobs, mode, true, st)) return JPEGQS_ERR_CUDA;
 			}
 			/* halo rows from the neighbours; the first exchange of a phase also ORs the flags */
 			if ((!xp.empty() || iter == 0) && slab_exchange(ctx, link, xp, bad_dev, iter == 0 ? nc : 0, st)) return JPEGQS_ERR_CUDA;
@@ -1627,22 +1615,15 @@ static int run_slab(jpegqs_cuda_ctx *ctx, jpegqs_cuda_link *link, jpegqs_cuda_im
 				for (CompWork *w : works) {
 					if (iter >= w->niter2) continue;
 					if (((iter == w->niter2 - 1 && !w->extra) ? 1 : 0) != clampv) continue;
-					jobs.push_back(make_job(*w, p2_of(w)));
+					jobs.push_back(slab_job(*w, plane2_of(s, *w, flags)));
 				}
 				if (jobs.empty()) continue;
-				const QsJob *jd; int tiles;
-				if (upload_jobs(ctx, 1, jobs, st, &jd, &tiles, true)) return JPEGQS_ERR_CUDA;
-				if (prof_begin(ctx, 1, st)) return JPEGQS_ERR_CUDA;
-				if (flags & QS_LOW_QUALITY) CK(qs_launch_lowq(jd, (int)jobs.size(), tiles, flags, clampv, bad_dev, st));
-				else CK(qs_launch_smooth(jd, (int)jobs.size(), tiles, tabs, tile_counter, flags, clampv, ctx->num_sms,
-						ctx->tune_sync, ctx->tune_wpg, bad_dev, st));
-				if (prof_end(ctx, st)) return JPEGQS_ERR_CUDA;
-				ctx->launches++;
+				if (launch_smooth(ctx, jobs, flags, clampv, true, st)) return JPEGQS_ERR_CUDA;
 			}
 		}
 		{	/* the component that overflowed is clamped only (2602-2610, 2670-2689); on the device */
 			std::vector<QsJob> jobs;
-			for (CompWork *w : works) jobs.push_back(make_job(*w, NULL));
+			for (CompWork *w : works) jobs.push_back(slab_job(*w, NULL));
 			if (!jobs.empty()) {
 				const QsJob *jd; int tiles;
 				if (upload_jobs(ctx, 0, jobs, st, &jd, &tiles, true)) return JPEGQS_ERR_CUDA;
@@ -1653,50 +1634,31 @@ static int run_slab(jpegqs_cuda_ctx *ctx, jpegqs_cuda_link *link, jpegqs_cuda_im
 		/* post steps: chroma up-sampling (2691-2752), luma planes (2753-2815); results are dropped
 		 * at the end if the run stopped */
 		for (CompWork *w : works) {
-			if (w->ci > 0 && image1 && w->ci <= 2) {
-				int ws = im->comp[0].h_samp, hs = im->comp[0].v_samp;
-				int w1 = ((int)im->image_width + ws - 1) / ws, h1 = ((int)im->image_height + hs - 1) / hs;
-				int W0 = im->comp[0].wblk, H0 = im->comp[0].hblk;
-				CK(qs_launch_upsample(w->plane, image2, QS_PLANE_STRIDE(w->W), image1, QS_PLANE_STRIDE(W0),
-						mem_buf[w->ci - 1], W0 * 8, w1, h1, ws, hs, W0 * 8, H0 * 8, (int)geom->row0[0] * 8, st));
-				CK(qs_launch_fdct_plane(mem_buf[w->ci - 1], W0 * 8, coef_up_dev[w->ci - 1], W0, H0, st));
-				ctx->launches += 2;
-			} else if (w->ci == 0 && need_ds) {
-				int ws = w->c->h_samp, hs = w->c->v_samp;
-				if (ws == 1 && hs == 1) image2 = w->plane;
+			if (w->ci > 0 && s.image1 && w->ci <= 2) {
+				if (post_upsample(ctx, s, *w, (int)geom->row0[0] * 8, st)) return JPEGQS_ERR_CUDA;
+			} else if (w->ci == 0 && s.need_downsample) {
+				if (w->c->h_samp == 1 && w->c->v_samp == 1) s.image2 = w->plane;
 				else {
-					if (flags & QS_UPSAMPLE_UV) image1 = w->plane;
-					const jpegqs_cuda_comp *cc = &im->comp[1];
-					int h = (int)geom->hblk_total[0] * 8, h2 = (int)geom->hblk_total[1] * 8, h1_total = (h + hs - 1) / hs;
-					int first = top ? -1 : (int)geom->row0[1] * 8;
-					int last = bottom ? h2 : (int)(geom->row0[1] + cc->hblk) * 8 - 1;
-					int dstride = QS_PLANE_STRIDE(cc->wblk);
-					if (last >= first) {
-						CK(qs_launch_downsample(w->plane, QS_PLANE_STRIDE(w->W), w->W * 8, h,
-								image2_buf + (size_t)(first - (int)geom->row0[1] * 8 + 1) * dstride, dstride, (int)cc->wblk * 8, h2,
-								ws, hs, (int)geom->row0[0] * 8, first, last - first + 1, h1_total, st));
-						ctx->launches++;
-					}
-					image2 = image2_buf;
-					std::vector<XchgPlane> xp; xp.push_back({ image2_buf, (int)cc->wblk, (int)cc->hblk });
+					if (flags & QS_UPSAMPLE_UV) s.image1 = w->plane;
+					if (post_downsample(ctx, s, *w, (int)geom->row0[0], (int)geom->hblk_total[0], (int)geom->row0[1],
+							(int)geom->hblk_total[1], top, bottom, st)) return JPEGQS_ERR_CUDA;
+					s.image2 = s.image2_buf;
+					std::vector<XchgPlane> xp; xp.push_back({ s.image2_buf, (int)im->comp[1].wblk, (int)im->comp[1].hblk });
 					if (slab_exchange(ctx, link, xp, bad_dev, 0, st)) return JPEGQS_ERR_CUDA;
 				}
 			}
 		}
 		if (!on_device) {                                                  /* downloads of this phase, band by band */
 			CK(cudaEventRecord(ctx->sync_ev[2 * g + 1], st));
+			const int H0 = (int)im->comp[0].hblk;
 			for (int k = 0; k < nbands[g]; k++) {
 				std::vector<IoSeg> segs;
 				for (int ci = c0; ci < c1; ci++) {
 					CompWork &w = W[ci];
 					int r0 = (int)((long)k * w.H / nbands[g]), r1 = (int)((long)(k + 1) * w.H / nbands[g]);
-					if (w.W && r1 > r0) segs.push_back(seg_of(w, r0, r1));
-					if (image1 && ci >= 1 && ci <= 2) {
-						int H0 = (int)im->comp[0].hblk;
-						IoSeg sg; sg.dev = coef_up_dev[ci - 1]; sg.pin = w.pin_up; sg.rows = w.rows_up;
-						sg.wblk = im->comp[0].wblk; sg.r0 = (int)((long)k * H0 / nbands[g]); sg.r1 = (int)((long)(k + 1) * H0 / nbands[g]);
-						if (sg.r1 > sg.r0) segs.push_back(sg);
-					}
+					if (w.W && r1 > r0) segs.push_back(coef_seg(w, r0, r1));
+					r0 = (int)((long)k * H0 / nbands[g]); r1 = (int)((long)(k + 1) * H0 / nbands[g]);
+					if (s.image1 && ci >= 1 && ci <= 2 && r1 > r0) segs.push_back(up_seg(s, w, r0, r1));
 				}
 				if (io.download(std::move(segs), ctx->sync_ev[2 * g + 1])) return JPEGQS_ERR_CUDA;
 			}
@@ -1704,24 +1666,20 @@ static int run_slab(jpegqs_cuda_ctx *ctx, jpegqs_cuda_link *link, jpegqs_cuda_im
 	}
 	CK(cudaEventRecord(ctx->ev1, st));
 	CK(qs_copy_flags(bad_dev, ctx->flags_host, nc, st));
-	CK(cudaStreamSynchronize(st));
-	if (!on_device && io.finish()) return JPEGQS_ERR_CUDA;
+	if (run_end(ctx, io, on_device, st)) return JPEGQS_ERR_CUDA;
 	if (link && *link->timeout_host) {
 		int *t = link->timeout_host;
 		snprintf(ctx->err, sizeof(ctx->err), "sharded run: rank %d of %d waited 10 s for %s %d: sequence %d expected, %d found "
-				"(its own count: %u)", rank, world, t[1] > 32 ? "the mask message of peer" : "the halo rows of neighbour", 
+				"(its own count: %u)", rank, world, t[1] > 32 ? "the mask message of peer" : "the halo rows of neighbour",
 				t[1] > 32 ? t[1] - 33 : t[1] - 1, t[2], t[3], link->seq);
 		memset(t, 0, 4 * sizeof(int));
 		return JPEGQS_ERR_TIMEOUT;
 	}
-	int stop = static_stop_ci < (1 << 30) ? 1 : 0;
+	int stop = s.stop;
 	for (int ci = 0; ci < nc; ci++) if (W[ci].iterate && ctx->flags_host[ci]) stop = 1;
 	/* NOTE on upsampled chroma when the run stopped: coef_up holds data nobody will look at */
-	for (int ci = 0; ci < nc; ci++) if (im->comp[ci].has_qtbl) for (int k = 0; k < 64; k++) im->comp[ci].quant[k] = 1;
-	im->upsampled = (image1 && !stop) ? 1 : 0;
+	image_finish(im, s.image1 && !stop);
 	if (ret) *ret = stop;
-	CK(cudaEventElapsedTime(&ctx->last_ms, ctx->ev0, ctx->ev1));
-	if (prof_collect(ctx)) return JPEGQS_ERR_CUDA;
 	return 0;
 }
 
@@ -1882,102 +1840,6 @@ extern "C" int jpegqs_cuda_run_host_multi(jpegqs_cuda_multi *m, jpegqs_cuda_imag
 	for (int c = 0; c < img->ncomp; c++) memcpy(img->comp[c].quant, slab[0].comp[c].quant, sizeof(img->comp[c].quant));
 	img->upsampled = slab[0].upsampled;
 	return out;
-}
-
-/* ------------------------------------------------------------------------------------------
- * pass-level entry points
- * ------------------------------------------------------------------------------------------ */
-static int stage_jobs(jpegqs_cuda_ctx *ctx, int njobs, const jpegqs_cuda_job *jobs, int slot, cudaStream_t st,
-		const QsJob **jd, int *tiles) {
-	if (njobs < 0 || njobs > QS_MAX_JOBS || (njobs && !jobs)) return JPEGQS_ERR_ARG;
-	CK(cudaSetDevice(ctx->device));
-	if (quant_reserve(ctx, QS_MAX_JOBS)) return JPEGQS_ERR_CUDA;
-	std::vector<QsQuantDev> q(njobs); std::vector<QsJob> v(njobs);
-	for (int i = 0; i < njobs; i++) {
-		int val; quant_prepare(jobs[i].quant, &q[i], &val, ctx->tune_maxn, ctx->tune_uni, ctx->tune_merge);
-		QsJob &j = v[i]; memset(&j, 0, sizeof(j));
-		j.coef = jobs[i].coef; j.plane = jobs[i].plane; j.plane2 = jobs[i].plane2;
-		j.quant = ctx->quant_dev + i;
-		j.wblk = jobs[i].wblk; j.hblk = jobs[i].hblk; j.stride = QS_PLANE_STRIDE(j.wblk);
-		j.nblocks = j.wblk * j.hblk; j.luma = jobs[i].luma;
-		j.top_edge = jobs[i].top_edge; j.bottom_edge = jobs[i].bottom_edge;
-	}
-	assign_sched_slots(q.data(), njobs);
-	if (njobs) CK(cudaMemcpyAsync(ctx->quant_dev, q.data(), njobs * sizeof(QsQuantDev), cudaMemcpyHostToDevice, st));
-	ctx->jobs_cache[slot].clear();
-	return upload_jobs(ctx, slot, v, st, jd, tiles);
-}
-
-extern "C" int jpegqs_cuda_pass_idct(jpegqs_cuda_ctx *ctx, int njobs, const jpegqs_cuda_job *jobs, int mode,
-		int *bad, void *stream) {
-	if (!ctx) return JPEGQS_ERR_ARG;
-	cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
-	const QsJob *jd; int tiles;
-	int rc = stage_jobs(ctx, njobs, jobs, 0, st, &jd, &tiles);
-	if (rc) return rc;
-	int m = ((mode & JPEGQS_PASS_DEQUANT) ? QS_IDCT_DEQUANT : 0) | ((mode & JPEGQS_PASS_CLAMP) ? QS_IDCT_CLAMP : 0);
-	CK(cudaMemsetAsync(ctx->flags_dev, 0, (njobs ? njobs : 1) * sizeof(int), st));
-	CK(qs_launch_idct_pass(jd, njobs, tiles, m, ctx->flags_dev, st));
-	if (bad) {
-		*bad = 0;
-		if (njobs) {
-			CK(qs_copy_flags(ctx->flags_dev, ctx->flags_host, njobs, st));
-			CK(cudaStreamSynchronize(st));
-			for (int i = 0; i < njobs; i++) if (ctx->flags_host[i]) *bad |= (int)(1u << (i < 31 ? i : 31));
-		}
-	}
-	return 0;
-}
-
-extern "C" int jpegqs_cuda_pass_smooth(jpegqs_cuda_ctx *ctx, int njobs, const jpegqs_cuda_job *jobs, int flags,
-		int clamp_out, void *stream) {
-	if (!ctx) return JPEGQS_ERR_ARG;
-	cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
-	const QsJob *jd; int tiles;
-	int rc = stage_jobs(ctx, njobs, jobs, 1, st, &jd, &tiles);
-	if (rc) return rc;
-	const float *tabs = (flags & QS_DIAGONALS) ? ctx->tab_diag : ctx->tab_plain;
-	if (flags & QS_LOW_QUALITY) CK(qs_launch_lowq(jd, njobs, tiles, flags, clamp_out, NULL, st));
-#ifdef QS_EXPERIMENTS
-	else if (ctx->tune_x2) CK(qs_launch_smooth_x2(jd, njobs, tiles, (flags & QS_DIAGONALS) ? ctx->tab2_diag : ctx->tab2_plain,
-			ctx->nslots2, ctx->flags_dev + QS_MAX_JOBS, flags, clamp_out, ctx->num_sms, ctx->tune_sync, st));
-#endif
-	else CK(qs_launch_smooth(jd, njobs, tiles, tabs, ctx->flags_dev + QS_MAX_JOBS, flags, clamp_out, ctx->num_sms, ctx->tune_sync, ctx->tune_wpg, NULL, st));
-	return 0;
-}
-
-/* ---- luma -> chroma hand-over for slabs (JOINT_YUV / UPSAMPLE_UV across GPUs) ------------- */
-extern "C" int jpegqs_cuda_pass_downsample(jpegqs_cuda_ctx *ctx, const uint8_t *yplane, uint32_t y_wblk,
-		uint32_t y_row0, uint32_t y_hblk_total, uint8_t *plane2, uint32_t c_wblk, uint32_t c_rows, uint32_t c_row0,
-		uint32_t c_hblk_total, int ws, int hs, int top_edge, int bottom_edge, void *stream) {
-	if (!ctx || !yplane || !plane2 || ws < 1 || hs < 1) return JPEGQS_ERR_ARG;
-	CK(cudaSetDevice(ctx->device));
-	cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
-	int h = (int)y_hblk_total * 8, h2 = (int)c_hblk_total * 8, h1_total = (h + hs - 1) / hs;
-	int first = top_edge ? -1 : (int)c_row0 * 8;
-	int last = bottom_edge ? h2 : (int)(c_row0 + c_rows) * 8 - 1;
-	int dstride = QS_PLANE_STRIDE(c_wblk);
-	if (last < first) return 0;
-	CK(qs_launch_downsample(yplane, QS_PLANE_STRIDE(y_wblk), (int)y_wblk * 8, h,
-			plane2 + (size_t)(first - (int)c_row0 * 8 + 1) * dstride, dstride, (int)c_wblk * 8, h2, ws, hs,
-			(int)y_row0 * 8, first, last - first + 1, h1_total, st));
-	return 0;
-}
-
-extern "C" int jpegqs_cuda_pass_upsample(jpegqs_cuda_ctx *ctx, const uint8_t *cplane, const uint8_t *plane2,
-		uint32_t c_wblk, const uint8_t *yplane, uint32_t y_wblk, uint32_t y_rows, uint32_t y_row0,
-		int16_t *coef_up, uint8_t *scratch, int ws, int hs, uint32_t image_width, uint32_t image_height,
-		void *stream) {
-	if (!ctx || !cplane || !plane2 || !yplane || !coef_up || !scratch || ws < 1 || hs < 1) return JPEGQS_ERR_ARG;
-	CK(cudaSetDevice(ctx->device));
-	cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
-	int w1 = ((int)image_width + ws - 1) / ws, h1 = ((int)image_height + hs - 1) / hs;
-	int ww = (int)y_wblk * 8, hh = (int)y_rows * 8;
-	if (!ww || !hh) return 0;
-	CK(qs_launch_upsample(cplane, plane2, QS_PLANE_STRIDE(c_wblk), yplane, QS_PLANE_STRIDE(y_wblk),
-			scratch, ww, w1, h1, ws, hs, ww, hh, (int)y_row0 * 8, st));
-	CK(qs_launch_fdct_plane(scratch, ww, coef_up, (int)y_wblk, (int)y_rows, st));
-	return 0;
 }
 
 /* ---- decode to RGB (SURVEY.md 8f row f2) --------------------------------------------------- */

@@ -43,19 +43,12 @@ class _Image(C.Structure):
                 ("comp", _Comp * MAX_COMP), ("upsampled", C.c_int32)]
 
 
-class _Job(C.Structure):
-    _fields_ = [("coef", C.c_void_p), ("plane", C.c_void_p), ("plane2", C.c_void_p),
-                ("wblk", C.c_uint32), ("hblk", C.c_uint32), ("quant", C.c_uint16 * 64),
-                ("luma", C.c_int32), ("top_edge", C.c_int32), ("bottom_edge", C.c_int32)]
-
-
 class _Slab(C.Structure):
     _fields_ = [("rank", C.c_int32), ("world", C.c_int32),
                 ("row0", C.c_uint32 * MAX_COMP), ("hblk_total", C.c_uint32 * MAX_COMP)]
 
 
 PROGRESS_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_int, C.c_int)
-PASS_DEQUANT, PASS_CLAMP = 1, 2
 
 _lib = None
 
@@ -91,16 +84,6 @@ def load():
     lib.jpegqs_cuda_plane_bytes.argtypes = [C.c_uint32, C.c_uint32]
     lib.jpegqs_cuda_plane_bytes.restype = C.c_size_t
     lib.jpegqs_cuda_plane_stride.argtypes = [C.c_uint32]
-    lib.jpegqs_cuda_pass_idct.argtypes = [C.c_void_p, C.c_int, C.POINTER(_Job), C.c_int,
-                                          C.POINTER(C.c_int), C.c_void_p]
-    lib.jpegqs_cuda_pass_smooth.argtypes = [C.c_void_p, C.c_int, C.POINTER(_Job), C.c_int, C.c_int,
-                                            C.c_void_p]
-    lib.jpegqs_cuda_pass_downsample.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32,
-                                                C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32,
-                                                C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]
-    lib.jpegqs_cuda_pass_upsample.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p,
-                                              C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p,
-                                              C.c_int, C.c_int, C.c_uint32, C.c_uint32, C.c_void_p]
     lib.jpegqs_cuda_render_rgb.argtypes = [C.c_void_p, C.POINTER(_Image), C.c_int, C.c_void_p, C.c_void_p]
     lib.jpegqs_cuda_set_profiling.argtypes = [C.c_void_p, C.c_int]
     lib.jpegqs_cuda_kernel_stats.argtypes = [C.c_void_p, C.POINTER(C.c_float), C.POINTER(C.c_int),
@@ -397,42 +380,6 @@ class QsContext:
                 if c.quant is not None:
                     c.quant = np.array(list(ci.comp[i].quant), dtype=np.uint16)
         return ret, bool(ci.upsampled), up_arrays
-
-    # ---- pass level (multi-GPU slabs) ----
-    @staticmethod
-    def make_job(coef_ptr, plane_ptr, plane2_ptr, wblk, hblk, quant, luma, top_edge, bottom_edge) -> _Job:
-        j = _Job()
-        j.coef, j.plane, j.plane2 = coef_ptr, plane_ptr, plane2_ptr or None
-        j.wblk, j.hblk = wblk, hblk
-        for k in range(64):
-            j.quant[k] = int(quant[k])
-        j.luma, j.top_edge, j.bottom_edge = int(luma), int(top_edge), int(bottom_edge)
-        return j
-
-    def pass_idct(self, jobs: List[_Job], mode: int, want_bad: bool = False, stream: int = 0) -> int:
-        arr = (_Job * len(jobs))(*jobs)
-        bad = C.c_int(0)
-        self._check(self.lib.jpegqs_cuda_pass_idct(self.h, len(jobs), arr, mode,
-                                                   C.byref(bad) if want_bad else None,
-                                                   C.c_void_p(stream or None)))
-        return bad.value
-
-    def pass_smooth(self, jobs: List[_Job], flags: int, clamp_out: bool, stream: int = 0):
-        arr = (_Job * len(jobs))(*jobs)
-        self._check(self.lib.jpegqs_cuda_pass_smooth(self.h, len(jobs), arr, flags & 0x7f, int(clamp_out),
-                                                     C.c_void_p(stream or None)))
-
-    def pass_downsample(self, yplane, y_wblk, y_row0, y_hblk_total, plane2, c_wblk, c_rows, c_row0,
-                        c_hblk_total, ws, hs, top_edge, bottom_edge, stream: int = 0):
-        self._check(self.lib.jpegqs_cuda_pass_downsample(
-            self.h, yplane, y_wblk, y_row0, y_hblk_total, plane2, c_wblk, c_rows, c_row0, c_hblk_total,
-            ws, hs, int(top_edge), int(bottom_edge), C.c_void_p(stream or None)))
-
-    def pass_upsample(self, cplane, plane2, c_wblk, yplane, y_wblk, y_rows, y_row0, coef_up, scratch,
-                      ws, hs, image_width, image_height, stream: int = 0):
-        self._check(self.lib.jpegqs_cuda_pass_upsample(
-            self.h, cplane, plane2, c_wblk, yplane, y_wblk, y_rows, y_row0, coef_up, scratch, ws, hs,
-            image_width, image_height, C.c_void_p(stream or None)))
 
     def plane_bytes(self, wblk, hblk) -> int:
         return int(self.lib.jpegqs_cuda_plane_bytes(wblk, hblk))

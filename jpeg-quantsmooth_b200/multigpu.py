@@ -1,34 +1,18 @@
-"""MCU-row sharding of one image across the GPUs of a box (SURVEY.md 8e) - the round-1 Python
-orchestration over the pass-level C ABI.  Since round 2 the product path is the C slab engine
-(csrc/qs_cuda.cu run_slab, include/jpegqs_cuda.h "one image sharded by MCU rows": kernel-side
-exchange over peer mailboxes, device-side stop logic); this module stays as the CPU-testable
-statement of the shard geometry and schedule (tests/test_multigpu_gloo.py drives it with oracle
-passes over gloo) and provides split_mcu_rows / comp_block_rows to bench.py and the tools.
+"""Geometry of an image sharded by MCU rows (SURVEY.md 8e), for callers that cut slabs
+themselves: bench.py's multi-GPU arm, tools/run_configs.py and the tests.
 
-One process per GPU (torch.distributed, NCCL over NVLink).  Every rank owns a contiguous
-range of MCU rows of every component.  Within an iteration blocks only need the
-previous-pass samples of the 1-pixel ring around them (reference quantsmooth.h:1396-1401,
-Jacobi structure), so the only exchange is ONE pixel row per component per slab boundary
-after every IDCT pass: a neighbour exchange (send/recv), not a collective.  JOINT_YUV /
-UPSAMPLE_UV add one more row exchange for the down-sampled luma plane handed from the luma
-phase to the chroma phase.  The IDCT is integer-deterministic, so the result is bit-identical
-to the single-GPU run for any shard count (tests/test_multigpu_gloo.py, tests/test_gpu_edge.py).
-
-`run_slab` is the slab-local restatement of the launch schedule in csrc/qs_cuda.cu::run_images
-(itself the reference driver, quantsmooth.h:2404-2878).  The pass implementation is
-pluggable: the product uses `CudaPasses` (the C ABI's pass-level entry points); the CPU tests
-drive the same sharding / exchange / stop logic with oracle passes.
+The sharded run itself is the C slab engine (csrc/qs_cuda.cu run_slab / run_host_multi,
+include/jpegqs_cuda.h "one image sharded by MCU rows").  Every rank owns a contiguous range of
+MCU rows of every component; slabs are MCU aligned, so the luma, chroma and down-sampled luma
+planes of a slab line up.  These functions state the same split as the engine's
+jpegqs_cuda_run_host_multi, and the plane geometry its kernels use (include/jpegqs_cuda.h
+jpegqs_cuda_plane_stride / _pad).
 """
 from __future__ import annotations
 
-from dataclasses import dataclass
-from typing import List, Optional, Sequence, Tuple
+from typing import List, Tuple
 
-import numpy as np
-
-PASS_DEQUANT, PASS_CLAMP = 1, 2
 PLANE_PAD = 16
-F_DIAGONALS, F_JOINT_YUV, F_UPSAMPLE_UV, F_LOW_QUALITY = 1, 2, 4, 8
 
 
 def plane_stride(wblk: int) -> int:
@@ -50,222 +34,3 @@ def comp_block_rows(mcu_range: Tuple[int, int], v_samp: int, hblk: int) -> Tuple
     """Block rows of a component covered by an MCU-row range (libjpeg geometry: the last
     MCU row may be only partly present, image.blocks_for)."""
     return min(mcu_range[0] * v_samp, hblk), min(mcu_range[1] * v_samp, hblk)
-
-
-@dataclass(eq=False)
-class SlabComp:
-    coef: object            # tensor int16 [rows, wblk, 64] on the pass backend's device
-    plane: object           # tensor uint8 [rows*8+2, stride]
-    wblk: int
-    rows: int               # block rows in this slab
-    quant: np.ndarray       # raw quantval [64]
-    luma: bool
-    h_samp: int = 1
-    v_samp: int = 1
-    row0: int = 0           # first block row of the slab inside the whole component
-    hblk_total: int = 0     # block rows of the whole component (0: = rows, single slab)
-    plane2: object = None   # down-sampled luma plane handed to chroma components (JOINT_YUV)
-    coef_up: object = None  # out: tensor int16 [luma rows, luma wblk, 64] after UPSAMPLE_UV
-
-
-@dataclass
-class SlabGeom:
-    """The image-level fields do_quantsmooth reads (quantsmooth.h:2447-2453, 2694-2697)."""
-    is_ycbcr: bool
-    image_width: int
-    image_height: int
-
-
-class CudaPasses:
-    """Pass backend over the C ABI (jpegqs_cuda_pass_*)."""
-
-    def __init__(self, ctx, stream: int = 0):
-        # stream: a cudaStream_t handle.  0 is mapped to cudaStreamLegacy (0x1) so that the
-        # passes are ordered with torch work on the default stream; the C ABI reserves NULL
-        # for "the context's own stream".
-        self.ctx, self.stream = ctx, (stream or 1)
-
-    def _jobs(self, comps, top_edge, bottom_edge):
-        idx = [i for i, c in enumerate(comps) if c.rows]
-        jobs = [self.ctx.make_job(comps[i].coef.data_ptr(), comps[i].plane.data_ptr(),
-                                  comps[i].plane2.data_ptr() if comps[i].plane2 is not None else None,
-                                  comps[i].wblk, comps[i].rows, comps[i].quant, comps[i].luma,
-                                  top_edge, bottom_edge) for i in idx]
-        return idx, jobs
-
-    def idct(self, comps, mode, top_edge, bottom_edge, want_bad):
-        """Returns a bit mask over `comps` (bit i = comps[i] had an out-of-range coefficient)."""
-        idx, jobs = self._jobs(comps, top_edge, bottom_edge)
-        if not jobs:
-            return 0
-        m = self.ctx.pass_idct(jobs, mode, want_bad, self.stream)
-        return sum(1 << idx[k] for k in range(len(idx)) if (m >> min(k, 31)) & 1)
-
-    def smooth(self, comps, flags, clamp_out, top_edge, bottom_edge):
-        _, jobs = self._jobs(comps, top_edge, bottom_edge)
-        if jobs:
-            self.ctx.pass_smooth(jobs, flags, clamp_out, self.stream)
-
-    def clamp(self, comps):
-        for c in comps:
-            c.coef.clamp_(-1023, 1023)
-
-    def dequantize(self, c):
-        import torch
-        q = torch.as_tensor(np.asarray(c.quant, dtype=np.int32), device=c.coef.device)
-        c.coef.copy_((c.coef.to(torch.int32) * q).to(torch.int16))
-
-    def new_plane(self, like, rows, wblk):
-        import torch
-        return torch.zeros((rows * 8 + 2, plane_stride(wblk)), dtype=torch.uint8, device=like.device)
-
-    def downsample(self, y: SlabComp, c: SlabComp, plane2, ws, hs, top_edge, bottom_edge):
-        self.ctx.pass_downsample(y.plane.data_ptr(), y.wblk, y.row0, y.hblk_total or y.rows, plane2.data_ptr(),
-                                 c.wblk, c.rows, c.row0, c.hblk_total or c.rows, ws, hs, top_edge, bottom_edge,
-                                 self.stream)
-
-    def upsample(self, c: SlabComp, y: SlabComp, ws, hs, geom: SlabGeom):
-        import torch
-        c.coef_up = torch.empty((y.rows, y.wblk, 64), dtype=torch.int16, device=y.coef.device)
-        scratch = torch.empty((max(y.rows * 8, 1), y.wblk * 8), dtype=torch.uint8, device=y.coef.device)
-        self.ctx.pass_upsample(c.plane.data_ptr(), c.plane2.data_ptr(), c.wblk, y.plane.data_ptr(), y.wblk,
-                               y.rows, y.row0, c.coef_up.data_ptr(), scratch.data_ptr(), ws, hs,
-                               geom.image_width, geom.image_height, self.stream)
-        self._keep = scratch                     # alive until the stream has consumed it
-
-
-def make_flag_allreduce(dist, device):
-    """Returns f(bitmask) -> bitwise OR of the 32-bit mask over all ranks.  NCCL has no BOR,
-    so the mask travels as 32 0/1 lanes reduced with MAX."""
-    import torch
-    lanes = torch.zeros(32, dtype=torch.int32, device=device)
-    weights = [1 << i for i in range(32)]
-
-    def f(mask: int) -> int:
-        mask &= 0xFFFFFFFF
-        lanes.copy_(torch.tensor([(mask >> i) & 1 for i in range(32)], dtype=torch.int32))
-        dist.all_reduce(lanes, op=dist.ReduceOp.MAX)
-        got = lanes.cpu().tolist()
-        return sum(w for w, g in zip(weights, got) if g)
-    return f
-
-
-def exchange_rows(planes: Sequence[Tuple[object, int]], rank: int, world: int, dist, group=None):
-    """planes: (plane tensor, block rows).  Fills row 0 / row h+1 of every plane with the
-    neighbour slab's adjacent pixel row (side border bytes included).  The image's own
-    top/bottom rows are replicated by the passes.  Ranks holding no rows of a plane (more ranks
-    than MCU rows) are not supported by this simple neighbour scheme."""
-    if world == 1 or dist is None:
-        return
-    ops = []
-    for plane, rows in planes:
-        if not rows:
-            raise ValueError("sharded run: a rank holds no block row of a component (more ranks than MCU rows); "
-                             "use fewer ranks - the C engine's jpegqs_cuda_multi_plan does")
-        h = rows * 8
-        if rank > 0:
-            ops.append(dist.P2POp(dist.isend, plane[1], rank - 1, group))
-            ops.append(dist.P2POp(dist.irecv, plane[0], rank - 1, group))
-        if rank < world - 1:
-            ops.append(dist.P2POp(dist.isend, plane[h], rank + 1, group))
-            ops.append(dist.P2POp(dist.irecv, plane[h + 1], rank + 1, group))
-    if ops:
-        for req in dist.batch_isend_irecv(ops):
-            req.wait()
-
-
-def exchange_halos(comps: Sequence[SlabComp], rank: int, world: int, dist, group=None):
-    exchange_rows([(c.plane, c.rows) for c in comps], rank, world, dist, group)
-
-
-def run_slab(passes, comps: Sequence[SlabComp], flags: int, niter: int, rank: int, world: int,
-             dist=None, allreduce_flag=None, geom: Optional[SlabGeom] = None):
-    """do_quantsmooth on one slab of MCU rows.  Returns (stop, upsampled): the reference's
-    return value and whether comps[1..2].coef_up replace the chroma arrays (2835-2849)."""
-    niter = max(0, min(int(niter), 100))                              # 2455-2456
-    top, bottom = rank == 0, rank == world - 1
-    joint = bool(flags & (F_JOINT_YUV | F_UPSAMPLE_UV))
-    need_ds = bool(joint and geom is not None and geom.is_ycbcr and len(comps) >= 3 and
-                   all(c.h_samp == 1 and c.v_samp == 1 for c in comps[1:3]))   # 2447-2453
-    if niter <= 0 and not ((flags & F_UPSAMPLE_UV) and need_ds):
-        return 0, False                                               # 2458
-    stop, stop_ci = 0, 1 << 30
-    image1 = image2 = None                                            # luma slab comp / plane2 tensor
-    groups = [[0], list(range(1, len(comps)))] if need_ds else [list(range(len(comps)))]
-    for g in groups:
-        work, info = [], {}
-        for ci in g:                                                  # per-component prelude, 2484-2566
-            c = comps[ci]
-            val = int(np.bitwise_or.reduce(np.asarray(c.quant, dtype=np.int64)))
-            extra = 1 if (image1 is not None or (ci == 0 and need_ds)) else 0     # 2495
-            n2 = 0 if val <= 1 else niter                             # 2501
-            if val >= 0x800 and not stop:
-                stop, stop_ci = 1, ci                                 # 2504
-            if n2 + extra == 0:
-                continue
-            if stop:
-                passes.dequantize(c)                                  # 2551-2566
-                continue
-            c.plane2 = image2 if (image2 is not None and (flags & F_JOINT_YUV) and ci > 0) else None
-            info[id(c)] = [ci, n2, extra, True, False]                # ci, niter2, extra, active, clamped
-            work.append(c)
-        pos = {id(c): k for k, c in enumerate(work)}
-        max_pass = max([info[id(c)][1] + info[id(c)][2] for c in work], default=0)
-        for it in range(max_pass):
-            act = [c for c in work if info[id(c)][3] and it < info[id(c)][1] + info[id(c)][2]]
-            if not act:
-                break
-            bad = 0
-            for clampv in (0, 1):                                     # IDCT pass, 2589-2620 (+ final clamp)
-                sub = [c for c in act if (it == info[id(c)][1]) == bool(clampv)]
-                if not sub:
-                    continue
-                m = passes.idct(sub, (PASS_DEQUANT if it == 0 else 0) | (PASS_CLAMP if clampv else 0),
-                                top, bottom, it == 0)
-                for k, c in enumerate(sub):
-                    if clampv:
-                        info[id(c)][4] = True
-                    if (m >> k) & 1:
-                        bad |= 1 << pos[id(c)]
-            if it == 0:
-                if allreduce_flag is not None:
-                    bad = allreduce_flag(bad)                         # OR across ranks, 2602-2610
-                for k, c in enumerate(work):                          # components run in order
-                    ci = info[id(c)][0]
-                    if stop and ci > stop_ci:
-                        info[id(c)][3] = False; info[id(c)][4] = True     # only de-quantized (the pass did it)
-                    elif (bad >> k) & 1:
-                        stop, stop_ci = 1, ci
-                        info[id(c)][3] = False                        # falls to the clamp below
-                act = [c for c in act if info[id(c)][3]]
-            exchange_halos(act, rank, world, dist)
-            for clampv in (0, 1):                                     # smoothing pass, 2627-2640
-                sub = [c for c in act if it < info[id(c)][1] and
-                       ((it == info[id(c)][1] - 1 and not info[id(c)][2]) == bool(clampv))]
-                if sub:
-                    passes.smooth(sub, flags, bool(clampv), top, bottom)
-                    if clampv:
-                        for c in sub:
-                            info[id(c)][4] = True
-        left = [c for c in work if not info[id(c)][4]]
-        if left:
-            passes.clamp(left)                                        # 2670-2689
-        for c in work:                                                # post steps
-            ci = info[id(c)][0]
-            if stop:
-                continue
-            if ci > 0 and image1 is not None and ci <= 2:             # 2691-2752
-                y = image1
-                passes.upsample(c, y, y.h_samp, y.v_samp, geom)
-            elif ci == 0 and need_ds:                                 # 2753-2815
-                ws, hs = c.h_samp, c.v_samp
-                if ws == 1 and hs == 1:
-                    image2 = c.plane
-                else:
-                    if flags & F_UPSAMPLE_UV:
-                        image1 = c
-                    cc = comps[1]
-                    image2 = passes.new_plane(c.plane, cc.rows, cc.wblk)
-                    passes.downsample(c, cc, image2, ws, hs, top, bottom)
-                    exchange_rows([(image2, cc.rows)], rank, world, dist)
-    return stop, bool(image1 is not None and not stop)

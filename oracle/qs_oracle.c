@@ -589,49 +589,3 @@ void qso_set_threads(int n) {
 	(void)n;
 #endif
 }
-
-/* ------------------------------------------------------------------------------------
- * Slab-level helpers for the multi-GPU tests (tests/oracle_passes.py): the luma -> chroma
- * hand-over of quantsmooth.h:2753-2815 (down-sample) and 2691-2752 (upsample_row + FDCT)
- * expressed on explicit planes with row offsets, so that a slab of MCU rows can be processed
- * on its own.  Pointers address pixel (0,0) of the SLAB; rows are numbered inside the whole
- * component.  Validated through shard-count invariance against qso_run.
- * ------------------------------------------------------------------------------------ */
-void qso_downsample_rows(const uint8_t *y00, int ystride, int w, int h, int y_row0_px,
-		uint8_t *d00, int dstride, int w2, int ws, int hs, int c_row0_px, int first_row, int nrows, int h1_total) {
-	int r, x, w1 = (w + ws - 1) / ws;
-	for (r = first_row; r < first_row + nrows; r++) for (x = -1; x <= w2; x++) {
-		int cx = x < 0 ? 0 : x > w1 - 1 ? w1 - 1 : x, cy = r < 0 ? 0 : r > h1_total - 1 ? h1_total - 1 : r;
-		int h2 = h - cy * hs, ww2 = w - cx * ws, xx, yy, sum = 0, div;
-		const uint8_t *p = y00 + (size_t)(cy * hs - y_row0_px) * ystride + cx * ws;
-		h2 = h2 < hs ? h2 : hs; ww2 = ww2 < ws ? ww2 : ws; div = ww2 * h2;
-		for (yy = 0; yy < h2; yy++) for (xx = 0; xx < ww2; xx++) sum += p[yy * ystride + xx];
-		d00[(ptrdiff_t)(r - c_row0_px) * dstride + x] = (uint8_t)((sum + div / 2) / div);
-	}
-}
-
-void qso_upsample_rows(const uint8_t *c00, const uint8_t *d00, int cstride, const uint8_t *y00, int ystride,
-		uint8_t *out, int ostride, int w1, int h1, int ws, int hs, int ww, int hh, int oy0) {
-	int ox, oy;
-	for (oy = 0; oy < hh; oy++) for (ox = 0; ox < ww; ox++) {
-		int sx = ox < w1 * ws - 1 ? ox : w1 * ws - 1;
-		int sy = (oy + oy0 < h1 * hs - 1 ? oy + oy0 : h1 * hs - 1) - oy0;
-		int x = sx / ws, y = (sy + oy0) / hs - oy0 / hs, a; int32_t sA, sB;
-		const uint8_t *pc = c00 + (ptrdiff_t)y * cstride + x, *pd = d00 + (ptrdiff_t)y * cstride + x;
-		float scale = regress_scale(pd, pc, cstride, &sA, &sB);
-		float offset = (float)pc[0] - (float)pd[0] * scale + 0.5f;
-		a = cvtt((float)y00[(ptrdiff_t)sy * ystride + sx] * scale + offset);
-		out[(size_t)oy * ostride + ox] = a < 0 ? 0 : a > 255 ? 255 : a;
-	}
-}
-
-void qso_fdct_plane(const uint8_t *px, int pstride, int16_t *coef, int W, int H) {
-	int bx, by, x, y;
-	for (by = 0; by < H; by++) for (bx = 0; bx < W; bx++) {
-		float fb[64]; int16_t *cf = coef + ((size_t)by * W + bx) * 64;
-		for (y = 0; y < 8; y++) for (x = 0; x < 8; x++)
-			fb[y * 8 + x] = (float)(px[(size_t)(by * 8 + y) * pstride + bx * 8 + x] - 128);
-		qso_fdct_float(fb, fb);
-		for (x = 0; x < 64; x++) cf[x] = (int16_t)cvtt(roundf(fb[x]));
-	}
-}

@@ -1,5 +1,5 @@
-"""GPU edge cases, the libjpeg-facing C entry point, the batch and pass-level entry points,
-and size-independent properties at BASELINE.json's full sizes."""
+"""GPU edge cases, the libjpeg-facing C entry point, the batch entry point, and
+size-independent properties at BASELINE.json's full sizes."""
 import ctypes as C
 import hashlib
 
@@ -9,7 +9,6 @@ import pytest
 import jpegqs_b200 as qs
 import oracle_lib as ol
 from golden_io import adversarial_image, image_digest, reference_output
-from jpegqs_b200 import multigpu as mg
 
 pytestmark = pytest.mark.gpu
 
@@ -129,69 +128,6 @@ def test_batch_larger_than_one_launch(ctx):
         assert ol.images_equal(o, wants[i % 4])
 
 
-def _run_slabs_one_gpu(ctx, im, flags, niter, nshards):
-    """Emulates the multi-GPU schedule on one device: slabs are separate job sets, halo rows
-    are copied by hand between the IDCT and smoothing passes."""
-    import torch
-    dev = torch.device("cuda", 0)
-    vmax = max(c.v_samp for c in im.comps)
-    total = -(-im.height // (8 * vmax))
-    ranges = mg.split_mcu_rows(total, nshards)
-    slabs = []
-    for rng in ranges:
-        comps = []
-        for k, c in enumerate(im.comps):
-            r0, r1 = mg.comp_block_rows(rng, c.v_samp, c.hblk)
-            coef = torch.from_numpy(np.ascontiguousarray(c.coef[r0:r1])).to(dev)
-            plane = torch.zeros(((r1 - r0) * 8 + 2, mg.plane_stride(c.wblk)), dtype=torch.uint8, device=dev)
-            comps.append(mg.SlabComp(coef, plane, c.wblk, r1 - r0, c.quant, k == 0))
-        slabs.append(comps)
-    passes = mg.CudaPasses(ctx, torch.cuda.current_stream().cuda_stream)
-    for it in range(niter):
-        for r, comps in enumerate(slabs):
-            passes.idct(comps, mg.PASS_DEQUANT if it == 0 else 0, r == 0, r == nshards - 1, False)
-        for r in range(nshards - 1):
-            for a, b in zip(slabs[r], slabs[r + 1]):
-                if a.rows and b.rows:
-                    b.plane[0].copy_(a.plane[a.rows * 8])
-                    a.plane[a.rows * 8 + 1].copy_(b.plane[1])
-        for r, comps in enumerate(slabs):
-            passes.smooth(comps, flags, it == niter - 1, r == 0, r == nshards - 1)
-    torch.cuda.synchronize()
-    return [np.concatenate([s[k].coef.cpu().numpy() for s in slabs], axis=0) for k in range(len(im.comps))]
-
-
-@pytest.mark.parametrize("nshards,flags", [(2, 0), (3, 1), (5, 0), (3, 8)])
-def test_pass_level_slabs_are_shard_invariant(ctx, nshards, flags):
-    im = qs.synth.make_image(256, 208, "420")
-    got = _run_slabs_one_gpu(ctx, im, flags, 2, nshards)
-    _, want = ol.run_oracle(im, flags, 2)
-    for g, c in zip(got, want.comps):
-        assert np.array_equal(g, c.coef)
-
-
-@pytest.mark.parametrize("flags,ss,w,h", [(3, "420", 256, 208), (7, "420", 250, 130), (15, "420", 128, 96),
-                                          (7, "444", 96, 64), (7, "422", 128, 64)])
-def test_run_slab_pass_level_luma_chroma_handover(ctx, flags, ss, w, h):
-    """The pass-level path incl. jpegqs_cuda_pass_downsample / _upsample (one slab = the whole
-    image) against the oracle; the multi-slab logic on top is covered over gloo on the CPU."""
-    import torch
-    dev = torch.device("cuda", 0)
-    im = qs.synth.make_image(w, h, ss)
-    comps = [mg.SlabComp(torch.from_numpy(np.ascontiguousarray(c.coef)).to(dev),
-                         torch.zeros((c.hblk * 8 + 2, mg.plane_stride(c.wblk)), dtype=torch.uint8, device=dev),
-                         c.wblk, c.hblk, c.quant, k == 0, c.h_samp, c.v_samp, 0, c.hblk)
-             for k, c in enumerate(im.comps)]
-    passes = mg.CudaPasses(ctx, torch.cuda.current_stream().cuda_stream)
-    stop, ups = mg.run_slab(passes, comps, flags, 2, 0, 1, None, None, mg.SlabGeom(True, w, h))
-    torch.cuda.synchronize()
-    oret, want = ol.run_oracle(im, flags, 2)
-    assert stop == oret
-    for k, (c, o) in enumerate(zip(comps, want.comps)):
-        got = (c.coef_up if ups and k in (1, 2) else c.coef).cpu().numpy()
-        assert got.shape == o.coef.shape and np.array_equal(got, o.coef), k
-
-
 DEFAULT_MERGE = 1        # csrc/qs_cuda.cu tune_merge
 
 
@@ -251,12 +187,16 @@ def test_8k_q3_properties_and_row_band_parity(ctx):
         assert np.array_equal(c.coef[r0 + m:r0 + b.hblk - m], b.coef[m:b.hblk - m]), k
 
 
-def test_8k_q3_shard_invariance(ctx):
+def test_8k_q3_shard_invariance_over_processes(ctx):
+    """The headline shape over 4 ranks of the C slab engine, one process per rank (sharing
+    devices on a box with fewer GPUs, connected through CUDA IPC), against the single-device run."""
+    from test_gpu_slab_engine import run_ranks_in_processes
     im = qs.synth.make_image(7680, 4320, "420")
-    _, out = ctx.do_quantsmooth(im, 0, 3)
-    got = _run_slabs_one_gpu(ctx, im, 0, 3, 4)
-    for g, c in zip(got, out.comps):
-        assert np.array_equal(g, c.coef)
+    _, want = ctx.do_quantsmooth(im, 0, 3)
+    got = run_ranks_in_processes(4, 7680, 4320, "420", 0, 3, 1)
+    assert all(got[r][0][0] == 0 for r in range(4))
+    for k, c in enumerate(want.comps):
+        assert np.array_equal(np.concatenate([got[r][0][2][k] for r in range(4)], axis=0), c.coef), k
 
 
 def test_8k_q6_properties(ctx):

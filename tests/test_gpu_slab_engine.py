@@ -1,7 +1,7 @@
-"""The C slab engine (qs_cuda.cu run_slab / links / jpegqs_cuda_run_host_multi): one image cut
-into MCU-row slabs, halo rows and out-of-range masks exchanged by CUDA kernels through peer
-mailboxes, the reference's `stop` logic evaluated on the device.  Everything is compared with
-the ORACLE (never with the product's own single-GPU run).
+"""The C slab engine (qs_cuda.cu run_slab / links / jpegqs_cuda_run_host_multi), the only
+sharded path: one image cut into MCU-row slabs, halo rows and out-of-range masks exchanged by
+CUDA kernels through peer mailboxes, the reference's `stop` logic evaluated on the device.
+Everything is compared with the ORACLE (never with the product's own single-GPU run).
 
 A box with one GPU still runs the whole exchange: several ranks may share a device (contexts
 of one process connected "locally", or two processes connected through CUDA IPC handles)."""
@@ -60,7 +60,8 @@ def ctx():
 
 CASES = [(200, 136, "420", 0, 3), (200, 136, "420", 1, 2), (256, 200, "420", 3, 2), (256, 200, "420", 7, 3),
          (250, 130, "444", 7, 2), (160, 400, "gray", 1, 3), (136, 120, "422", 3, 2), (136, 120, "440", 0, 3),
-         (200, 136, "420", 8, 2), (200, 136, "420", 8 | 7, 1), (90, 50, "420", 7, 2), (200, 136, "420", 16, 2)]
+         (200, 136, "420", 8, 2), (200, 136, "420", 8 | 7, 1), (90, 50, "420", 7, 2), (200, 136, "420", 16, 2),
+         (128, 64, "422", 7, 2), (48, 40, "gray", 16, 3)]
 
 
 @pytest.mark.parametrize("w,h,ss,flags,niter", CASES)
@@ -91,21 +92,41 @@ def _devices(n):
     return [k % have for k in range(n)]       # ranks share devices when the box has fewer
 
 
+def _multi(world):
+    os.environ["JPEGQS_MIN_BLOCKS_PER_GPU"] = "1"                 # shard even tiny images
+    try:
+        return qs.cuda.QsMulti(_devices(world))
+    finally:
+        del os.environ["JPEGQS_MIN_BLOCKS_PER_GPU"]
+
+
+def _multi_matches_oracle(m, im, flags, niter):
+    ret, out = m.do_quantsmooth(im, flags, niter)
+    oret, want = ol.run_oracle(im, flags, niter)
+    assert ret == oret
+    assert ol.images_equal(out, want), f"{ol.diff_count(out, want)} coefficients differ"
+
+
 @pytest.mark.parametrize("world", [2, 3])
 @pytest.mark.parametrize("w,h,ss,flags,niter", CASES)
 def test_run_host_multi_matches_oracle(world, w, h, ss, flags, niter):
-    os.environ["JPEGQS_MIN_BLOCKS_PER_GPU"] = "1"                 # shard even tiny images
-    try:
-        m = qs.cuda.QsMulti(_devices(world))
-    finally:
-        del os.environ["JPEGQS_MIN_BLOCKS_PER_GPU"]
+    m = _multi(world)
     try:
         im = qs.synth.make_image(w, h, ss)
         assert m.plan(im) == world
-        ret, out = m.do_quantsmooth(im, flags, niter)
-        oret, want = ol.run_oracle(im, flags, niter)
-        assert ret == oret
-        assert ol.images_equal(out, want), f"{ol.diff_count(out, want)} coefficients differ"
+        _multi_matches_oracle(m, im, flags, niter)
+    finally:
+        m.close()
+
+
+@pytest.mark.parametrize("world,flags", [(2, 0), (3, 1), (5, 0), (3, 8)])
+def test_slabs_are_shard_invariant(world, flags):
+    """13 MCU rows over up to 5 ranks: slabs of 2 and 3 MCU rows, up to four interior boundaries."""
+    m = _multi(world)
+    try:
+        im = qs.synth.make_image(256, 208, "420")
+        assert m.plan(im) == world
+        _multi_matches_oracle(m, im, flags, 2)
     finally:
         m.close()
 
@@ -114,11 +135,7 @@ def test_run_host_multi_matches_oracle(world, w, h, ss, flags, niter):
 def test_multi_stop_reaches_every_rank(flags, niter):
     """An out-of-range coefficient in the LAST rank's slab: the first rank must leave that
     component alone as well (quantsmooth.h:2602-2610), which it only learns from the exchange."""
-    os.environ["JPEGQS_MIN_BLOCKS_PER_GPU"] = "1"
-    try:
-        m = qs.cuda.QsMulti(_devices(3))
-    finally:
-        del os.environ["JPEGQS_MIN_BLOCKS_PER_GPU"]
+    m = _multi(3)
     try:
         for comp, pos in ((0, -1), (1, -1), (2, 0), (1, 0)):
             im = qs.synth.make_image(160, 240, "420")
@@ -149,7 +166,7 @@ def test_multi_keeps_small_images_on_one_device():
 
 
 # ---- ranks in different processes: CUDA IPC mailboxes -------------------------------------------
-def _ipc_rank(rank, world, w, h, ss, flags, niter, conns, result):
+def _ipc_rank(rank, world, w, h, ss, flags, niter, reps, conns, result):
     import torch
     dev = rank % torch.cuda.device_count()
     ctx = qs.cuda.QsContext(dev)
@@ -165,7 +182,7 @@ def _ipc_rank(rank, world, w, h, ss, flags, niter, conns, result):
         handles[src] = c.recv()
     link.connect_ipc(handles)
     outs = []
-    for rep in range(2):                              # twice: sequence numbers carry over between runs
+    for rep in range(reps):
         s = slab.clone()
         ret, ups_flag, ups = ctx.run_slab(link, s, rank, world, row0, [c.hblk for c in im.comps], flags, niter)
         outs.append((ret, ups_flag, [c.coef for c in s.comps], ups))
@@ -174,15 +191,16 @@ def _ipc_rank(rank, world, w, h, ss, flags, niter, conns, result):
     ctx.close()
 
 
-@pytest.mark.parametrize("w,h,ss,flags,niter", [(320, 272, "420", 0, 3), (320, 272, "420", 7, 2), (256, 200, "444", 1, 2)])
-def test_two_processes_over_cuda_ipc(w, h, ss, flags, niter):
-    world = 2
+def run_ranks_in_processes(world, w, h, ss, flags, niter, reps):
+    """One process per rank (sharing devices on a box with fewer GPUs), mailboxes connected through
+    CUDA IPC handles.  Returns {rank: [(ret, upsampled, coefs, up arrays) per repetition]}."""
     sp = mp.get_context("spawn")
     pipes = {(a, b): sp.Pipe(duplex=False) for a in range(world) for b in range(world) if a != b}
     conns = [{"out": [pipes[(r, d)][1] for d in range(world) if d != r],
               "in": [(s, pipes[(s, r)][0]) for s in range(world) if s != r]} for r in range(world)]
     result = sp.Queue()
-    procs = [sp.Process(target=_ipc_rank, args=(r, world, w, h, ss, flags, niter, conns, result)) for r in range(world)]
+    procs = [sp.Process(target=_ipc_rank, args=(r, world, w, h, ss, flags, niter, reps, conns, result))
+             for r in range(world)]
     for p in procs:
         p.start()
     got = {}
@@ -192,6 +210,13 @@ def test_two_processes_over_cuda_ipc(w, h, ss, flags, niter):
     for p in procs:
         p.join(60)
         assert p.exitcode == 0
+    return got
+
+
+@pytest.mark.parametrize("w,h,ss,flags,niter", [(320, 272, "420", 0, 3), (320, 272, "420", 7, 2), (256, 200, "444", 1, 2)])
+def test_two_processes_over_cuda_ipc(w, h, ss, flags, niter):
+    world = 2
+    got = run_ranks_in_processes(world, w, h, ss, flags, niter, 2)   # twice: sequence numbers carry over
     im = qs.synth.make_image(w, h, ss)
     oret, want = ol.run_oracle(im, flags, niter)
     for rep in range(2):
